@@ -2,6 +2,7 @@
 """bench.py -- scenes/sec of the 3D-SIS dense-voxel TEST forward on B200 (BASELINE.json metric).
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--config cfg2|cfg3|cfg3s|cfg4|cfg5]
+                  [--dump-outputs DIR]
 
 A step = one pass of the hot path (back-projection -> 3D backbone -> RPN/NMS -> RoI pool + classifier -> per-RoI mask
 head) over a batch of synthetic scenes; ENet-shaped 2D features are an input (ENet is upstream of the path, SURVEY 8f2).
@@ -199,33 +200,10 @@ class Clocks:
 
 # ------------------------------------------------------------------------------------------------ CPU arm
 def reference_runner(wl):
-    """The reference's own CPU implementation of the path, best available: the UNMODIFIED reference Python files from
-    git-ignored baseline/_ref/ (copied there by __graft_entry__.build() while /root/reference is present; they travel to the
-    GPU box with the snapshot) driven by oracle/ref_harness.py with the SURVEY 8(c) shims -- kind "reference"; else the
-    oracle port -- kind "port".  Returns (kind, run(seed, dims, n_img) -> seconds of one full forward)."""
+    """The CPU implementation of the path: the torch-CPU oracle port of the reference (oracle/port.py, pinned to the
+    unmodified reference by tests/test_oracle_golden.py) -- kind "port".  Returns (kind, run(seed, dims, n_img) -> seconds
+    of one full forward)."""
     import sis3d_synth as synth
-    ref_root = os.path.join(ROOT, "baseline", "_ref")
-    yml = ("SUNCG" if wl["cfgname"] == "suncg" else "ScanNet") + "/rpn_class_mask_5.yml"
-    if os.path.isdir(os.path.join(ref_root, "lib", "nets")) and os.environ.get("SIS3D_CPU_ARM", "reference") == "reference":
-        try:
-            os.environ["SIS3D_REFERENCE"] = ref_root
-            sys.path.insert(0, os.path.join(ROOT, "oracle"))
-            import ref_harness as rh
-            cfg = rh.load_cfg(yml, USE_IMAGES=True, USE_IMAGES_GT=True, USE_MASK=True)
-            w = synth.make_weights(seed=0, net=cfg.NET, use_images=True, num_classes=cfg.NUM_CLASSES, a1=cfg.NUM_ANCHORS_LEVEL1,
-                                   a2=cfg.NUM_ANCHORS_LEVEL2, use_mask=True)
-            net = rh.build_net(cfg, w)
-
-            def run(seed, dims, n_img):
-                data, boxes = synth.make_scene(seed, dims)
-                v = synth.make_views(seed, dims, n_img, boxes, intrinsic=np.array(cfg.INTRINSIC, dtype=np.float32))
-                t0 = time.perf_counter()
-                rh.reference_forward(net, cfg, data, v)
-                return time.perf_counter() - t0
-            run(7, (48, 32, 48), 2)  # proves the harness works on this box before it is chosen
-            return "reference", run
-        except Exception as e:  # fall back to the port, and say why
-            print(f"[bench] baseline/_ref unusable ({type(e).__name__}: {e}); using the oracle port", file=sys.stderr)
     from oracle import port
     ocfg = port.make_cfg(wl["cfgname"])
     w = synth.make_weights(seed=0, net=ocfg.NET, use_images=True, num_classes=ocfg.NUM_CLASSES, a1=ocfg.NUM_ANCHORS_LEVEL1,
@@ -261,8 +239,7 @@ def cpu_arm(wl, seconds, min_scenes=1, max_scenes=10 ** 9):
     ts, t0 = [], time.perf_counter()
     while len(ts) < min_scenes or (time.perf_counter() - t0 < seconds and len(ts) < max_scenes):
         ts.append(run(*wl["scenes"][len(ts) % len(wl["scenes"])]))
-    what = ("unmodified reference Python files (baseline/_ref) under the SURVEY 8(c) shims, torch-CPU fp32, projection on the "
-            "CPU (MAX_VOLUME=0 semantics)") if kind == "reference" else "torch-CPU fp32 oracle port of the reference path"
+    what = "torch-CPU fp32 oracle port of the reference path"
     return dict(value=1.0 / float(np.mean(ts)), unit="scenes/s", cores=cores, kind=kind,
                 sample=f"{len(ts)} full forwards of the workload's scenes in {sum(ts):.0f}s, {what}"), ts
 
@@ -287,6 +264,30 @@ def run_reference(args, rank, wl):
 
 
 # ------------------------------------------------------------------------------------------------ GPU arm
+DUMP_BYTES = 64 * 10 ** 6
+
+
+def dump_outputs(out_dir, scenes):
+    """What the scene loop handed its caller for each scene of one step, in loop order, as the caller stores it
+    (lib/model/trainval.py save_scene_results): the [n, 16] detection table (box, score, class, mask keep, crop, count) and
+    the thresholded predicted-class mask of every kept detection.  float32 / float64 .npy files, DUMP_BYTES in all: mask
+    voxels beyond that are replaced by a fixed, seeded sample of them (mask_voxel_index)."""
+    os.makedirs(out_dir, exist_ok=True)
+    out = {"detections": np.concatenate([d for d, _, _ in scenes]).astype(np.float32),
+           "detections_per_scene": np.array([len(d) for d, _, _ in scenes], dtype=np.float64),
+           "masks_per_scene": np.array([0 if s is None else len(s) for _, _, s in scenes], dtype=np.float64),
+           "mask_sizes": np.concatenate([np.zeros((0, 3))] + [s for _, _, s in scenes if s is not None]).astype(np.float64)}
+    bits = np.concatenate([np.zeros(0, np.uint8)] + [b for _, b, _ in scenes if b is not None])
+    room = (DUMP_BYTES - 1024 * (len(out) + 2) - sum(a.nbytes for a in out.values())) // 4  # float32 slots; 1 KB per header
+    if bits.size > room:  # a sampled voxel costs 12 bytes: its value (float32) and its index (float64)
+        idx = np.sort(np.random.default_rng(0).choice(bits.size, room // 3, replace=False))
+        out["mask_voxel_index"] = idx.astype(np.float64)
+        bits = bits[idx]
+    out["mask_voxels"] = bits.astype(np.float32)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -301,7 +302,10 @@ def main():
     ap.add_argument("--cpu-baseline-seconds", type=float, default=20.0)
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--lean", action="store_true", help="profiling runs: timed loops only (no latency / parity / CPU legs)")
-    ap.add_argument("--host-profile", type=int, default=0, help="cProfile one pass -> gpurun_out/host_profile.txt")
+    ap.add_argument("--host-profile", type=int, default=0, help="cProfile one pass -> stderr")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step handed to its caller (rank 0: detection tables and thresholded "
+                         "masks of its scenes) as DIR/<name>.npy")
     args = ap.parse_args()
     rank, world = int(os.environ.get("RANK", 0)), int(os.environ.get("WORLD_SIZE", 1))
     local = int(os.environ.get("LOCAL_RANK", 0))
@@ -370,11 +374,12 @@ def main():
         e0.record()
         dets = []
         for _ in range(steps):
-            local_det = []
+            local_det, st["last"] = [], []
             for j, (_, P) in enumerate(net.forward_pipelined(inputs[k] for k in order)):
                 det = P["detections_host"]  # results of this scene are on the host: detection table + thresholded masks
                 d2h += det.nbytes + (P["mask_bits_host"].nbytes if "mask_bits_host" in P else 0)
                 dets.append(det)
+                st["last"].append((det, P.get("mask_bits_host"), P.get("mask_sizes")))
                 if mine is not None:
                     t = torch.from_numpy(det)
                     local_det.append((mine[j], t[:, :6], t[:, 7], t[:, 6]))
@@ -430,16 +435,17 @@ def main():
         wall = (time.perf_counter() - t0) / B * 1e3
         buf = io.StringIO()
         pstats.Stats(pr, stream=buf).sort_stats("tottime").print_stats(40)
-        os.makedirs(os.path.join(ROOT, "gpurun_out"), exist_ok=True)
-        with open(os.path.join(ROOT, "gpurun_out", "host_profile.txt"), "w") as f:
-            f.write(f"wall ms per scene (pipelined loop, host inputs, under cProfile): {wall:.3f}\n" + buf.getvalue())
+        print(f"wall ms per scene (pipelined loop, host inputs, under cProfile): {wall:.3f}\n" + buf.getvalue(), file=sys.stderr)
     clocks = Clocks(local)
     if rank == 0:
         clocks.start()
         time.sleep(0.3)
     ms_dev, launches, _, vox, nroi, nmask = timed_loop(dev_in, args.steps)
+    last_step = st["last"]
     ms_e2e, _, d2h, _, _, _ = timed_loop(host_in, args.steps)
     clock_summary = clocks.summary() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, last_step)
     n_scenes = args.steps * B  # scenes per rank inside each timed region
     total_scenes = n_scenes
     if world > 1:
@@ -640,8 +646,8 @@ def main():
                              "algorithmic_tflops": 0.894e6 * mvox / (mh * 1e-3) / 1e12,
                              "what": "ragged mask stage alone (plan + 6 layers + select) on 10 RoIs of 54x22x22, teacher-forced table"}
     if extras and not args.no_cpu_baseline:
-        # the reference's package is called `lib` like ours, so its CPU arm runs in a process of its own (the same code path as
-        # `--impl reference`); only if that fails is the in-process oracle port timed instead (kind "port")
+        # the CPU arm runs in a process of its own (the same code path as `--impl reference`); only if that fails is it timed
+        # in this process
         try:
             r = subprocess.run([sys.executable, os.path.abspath(__file__), "--impl", "reference", "--config", args.config,
                                 "--steps", "6", "--warmup", "1"], capture_output=True, text=True, timeout=400,

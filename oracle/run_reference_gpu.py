@@ -1,12 +1,13 @@
 #!/usr/bin/env python
 """oracle/run_reference_gpu.py -- TEST INFRASTRUCTURE (drop-in test of the operator boundary, SURVEY 8b).
 
-Runs the UNMODIFIED reference Python (network.py, proposal_layer.py, pth_nms.py, roi_pool.py, ... from git-ignored
-baseline/_ref/, staged there by __graft_entry__.build()) on the GPU in a process of its own -- the reference's package is
-called `lib`, like ours -- with its two cffi extension modules replaced by the ctypes stubs of INTEGRATION.md section 2 bound
-to libsis3d.so (oracle/ref_harness.py install(gpu=True)).  Writes the reference's _predictions for one named synthetic case.
+Runs the UNMODIFIED reference Python (network.py, proposal_layer.py, pth_nms.py, roi_pool.py, ... from the reference tree
+at $SIS3D_REFERENCE) on the GPU in a process of its own -- the reference's package is called `lib`, like ours -- with its
+two cffi extension modules replaced by the ctypes stubs of INTEGRATION.md section 2 bound to libsis3d.so
+(oracle/ref_harness.py install(gpu=True)).  Writes the reference's _predictions for one named synthetic case;
+oracle/make_golden_reference_gpu.py stores them as tests/golden/reference_gpu.npz.
 
-    python oracle/run_reference_gpu.py --case odd_45x27x41 --out /tmp/ref_gpu.npz
+    SIS3D_REFERENCE=<reference tree> python oracle/run_reference_gpu.py --case odd_45x27x41 --out ref_gpu.npz
 """
 import argparse
 import os
@@ -16,7 +17,6 @@ import numpy as np
 import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-os.environ.setdefault("SIS3D_REFERENCE", os.path.join(ROOT, "baseline", "_ref"))
 sys.path.insert(0, os.path.join(ROOT, "oracle"))
 SYNTH = os.path.join(ROOT, "3d-sis_b200", "sis3d_synth.py")
 

@@ -44,3 +44,31 @@ def test_other_configs_named_by_baseline():
     c5 = bench.workload("cfg5", 0, 8)
     assert c5["cfgname"] == "suncg" and c5["math_default"] == "fp16" and c5["scenes"][0][2] == 3
     assert abs(bench.alg_bytes((96, 48, 96), "suncg") - 729.3e6) < 1
+
+
+def test_dump_outputs_types_order_and_budget(tmp_path, monkeypatch):
+    """--dump-outputs: float32 / float64 files in loop order; above the byte budget the mask voxels become a seeded sample."""
+    rng = np.random.default_rng(0)
+    scenes = []
+    for n, sizes in ((3, [(2, 3, 4), (1, 1, 5)]), (2, None), (4, [(6, 2, 2)])):
+        det = rng.standard_normal((n, 16)).astype(np.float32)
+        if sizes is None:
+            scenes.append((det, None, None))
+        else:
+            sz = np.array(sizes, dtype=np.int32)
+            scenes.append((det, (rng.random(int(np.prod(sz, axis=1).sum())) > 0.5).astype(np.uint8), sz))
+    bench.dump_outputs(str(tmp_path / "all"), scenes)
+    got = {f[:-4]: np.load(tmp_path / "all" / f) for f in os.listdir(tmp_path / "all")}
+    assert all(a.dtype in (np.float32, np.float64) for a in got.values()) and "mask_voxel_index" not in got
+    assert np.array_equal(got["detections"], np.concatenate([d for d, _, _ in scenes]))
+    assert got["detections_per_scene"].tolist() == [3, 2, 4] and got["masks_per_scene"].tolist() == [2, 0, 1]
+    bits = np.concatenate([scenes[0][1], scenes[2][1]])
+    assert np.array_equal(got["mask_voxels"], bits) and got["mask_sizes"].tolist() == [[2, 3, 4], [1, 1, 5], [6, 2, 2]]
+    budget = sum(a.nbytes for k, a in got.items() if k != "mask_voxels") + 1024 * 6 + 4 * 30
+    monkeypatch.setattr(bench, "DUMP_BYTES", budget)
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), scenes)
+    idx, vals = np.load(tmp_path / "a" / "mask_voxel_index.npy"), np.load(tmp_path / "a" / "mask_voxels.npy")
+    assert len(idx) == 10 and np.array_equal(vals, bits[idx.astype(np.int64)])
+    assert np.array_equal(idx, np.load(tmp_path / "b" / "mask_voxel_index.npy"))
+    assert sum(os.path.getsize(tmp_path / "a" / f) for f in os.listdir(tmp_path / "a")) <= budget

@@ -1,32 +1,23 @@
 """Drop-in test of the operator boundary (SURVEY 8b, INTEGRATION.md section 2): the reference's OWN Python -- network.py,
-proposal_layer.py, pth_nms.py, roi_pool.py, unmodified, from git-ignored baseline/_ref/ -- runs on the GPU with its two cffi
-extension modules rebound to libsis3d.so (`gpu_nms` -> sis3d_nms, `roi_pooling_forward_cuda` -> sis3d_roi_pool_fwd), in a
-process of its own (oracle/run_reference_gpu.py).  Its predictions must equal (a) the CPU oracle, which is pinned to the
-all-CPU run of the same files, and (b) this repo's Network.forward on the same inputs."""
-import os
-import subprocess
-import sys
-
+proposal_layer.py, pth_nms.py, roi_pool.py, unmodified -- run on a B200 with its two cffi extension modules rebound to
+libsis3d.so (`gpu_nms` -> sis3d_nms, `roi_pooling_forward_cuda` -> sis3d_roi_pool_fwd) by oracle/run_reference_gpu.py.
+Its predictions are stored in tests/golden/reference_gpu.npz (generator: oracle/make_golden_reference_gpu.py) and must
+equal (a) the CPU oracle, which is pinned to the all-CPU run of the same files, and (b) this repo's Network.forward on the
+same inputs."""
 import numpy as np
 import pytest
 import torch
 
 import sis3d_synth as synth
-from conftest import ROOT
+from conftest import load_golden
 
 pytestmark = pytest.mark.gpu
 
 
 @pytest.mark.parametrize("tag", ["odd_45x27x41", "cfg1_32"])
-def test_reference_python_runs_over_libsis3d_extension_stubs(oracle, tag, tmp_path):
-    if not os.path.isdir(os.path.join(ROOT, "baseline", "_ref", "lib", "nets")):
-        pytest.skip("baseline/_ref not staged (python __graft_entry__.py build, in the container that has /root/reference)")
-    out = str(tmp_path / "ref_gpu.npz")
-    env = {k: v for k, v in os.environ.items() if k != "PYTHONPATH"}
-    r = subprocess.run([sys.executable, os.path.join(ROOT, "oracle", "run_reference_gpu.py"), "--case", tag, "--out", out],
-                       capture_output=True, text=True, timeout=900, env=env, cwd=str(tmp_path))
-    assert r.returncode == 0, r.stdout[-2000:] + r.stderr[-4000:]
-    ref = dict(np.load(out))
+def test_reference_python_runs_over_libsis3d_extension_stubs(oracle, tag):
+    g = load_golden("reference_gpu.npz")
+    ref = {k[len(f"dropin_{tag}_"):]: v for k, v in g.items() if k.startswith(f"dropin_{tag}_")}
     c = synth.CASES[tag]
     assert ref["convs_on_cuda"] == 1 and ref["gpu_nms_calls"] >= 1 and ref["roi_cuda_calls"] >= 1, "the rebound kernels must have run"
     ocfg, w, data, views = synth.build_case(oracle, c)

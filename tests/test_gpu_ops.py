@@ -57,28 +57,14 @@ def test_nms_edge_cases(oracle):
 
 
 def test_nms_mask_vs_reference_cuda_kernel(oracle):
-    """Bitmask of the reference's own kernel (compiled unmodified into oracle/_ref) == ours -> same keep."""
-    path = os.path.join(ROOT, "oracle", "_ref", "libref_nms_cuda.so")
-    if not os.path.exists(path):
-        pytest.skip("oracle/_ref not built")
-    ref = C.CDLL(path)
-    for seed, n, thr in ((0, 400, 0.1), (7, 777, 0.25)):
-        b = synth.make_nms_boxes(seed, n)
-        bd = torch.from_numpy(b).to(DEV)
-        cb = (n + 63) // 64
-        mask = torch.zeros(n, cb, dtype=torch.int64, device=DEV)
-        torch.cuda.synchronize()
-        ref._nms(C.c_int(n), C.c_void_p(bd.data_ptr()), C.c_void_p(mask.data_ptr()), C.c_float(thr))
-        torch.cuda.synchronize()
-        m = mask.cpu().numpy().view(np.uint64)
-        remv = np.zeros(cb, np.uint64)
-        keep = []
-        for i in range(n):  # host reduce of lib/layer_utils/nms/src/nms_cuda.c:41-59
-            if not (remv[i // 64] >> np.uint64(i % 64)) & np.uint64(1):
-                keep.append(i)
-                remv[i // 64:] |= m[i, i // 64:]
-        from lib.layer_utils.nms_wrapper import nms
-        assert nms(bd, thr).cpu().tolist() == keep
+    """Keep list of the reference's own kernel (its bitmask reduced as nms_cuda.c does; tests/golden/reference_gpu.npz,
+    generator oracle/make_golden_reference_gpu.py) == ours."""
+    from lib.layer_utils.nms_wrapper import nms
+    g = load_golden("reference_gpu.npz")
+    for seed in (0, 7):
+        s, n, thr = g[f"nms_cuda_cfg_{seed}"]
+        bd = torch.from_numpy(synth.make_nms_boxes(int(s), int(n))).to(DEV)
+        assert nms(bd, float(thr)).cpu().tolist() == g[f"nms_cuda_keep_{seed}"].tolist()
 
 
 # ---------------------------------------------------------------- RoI pooling
@@ -131,17 +117,9 @@ def test_roi_pool_golden_and_reference_cuda(oracle):
     fn = RoIPoolFunction(4, 4, 4, 0.25)
     out = fn(fd, rd)
     assert np.array_equal(out.cpu().numpy(), g["roi_out"])  # reference CPU C kernel
-    path = os.path.join(ROOT, "oracle", "_ref", "libref_roi_cuda.so")
-    if os.path.exists(path):
-        ref = C.CDLL(path)
-        top = torch.zeros_like(out)
-        arg = torch.zeros(out.shape, dtype=torch.int32, device=DEV)
-        torch.cuda.synchronize()
-        ref.ROIPoolForwardLaucher(C.c_void_p(fd.data_ptr()), C.c_float(0.25), rd.shape[0], 24, 12, 24, 16, 4, 4, 4,
-                                  C.c_void_p(rd.data_ptr()), C.c_void_p(top.data_ptr()), C.c_void_p(arg.data_ptr()),
-                                  C.c_void_p(0))
-        torch.cuda.synchronize()
-        assert torch.equal(top, out) and torch.equal(arg, fn.argmax)
+    ref = load_golden("reference_gpu.npz")  # reference CUDA kernel (generator: oracle/make_golden_reference_gpu.py)
+    assert np.array_equal(out.cpu().numpy(), ref["roi_cuda_top"].reshape(out.shape))
+    assert np.array_equal(fn.argmax.cpu().numpy(), ref["roi_cuda_argmax"].reshape(fn.argmax.shape))
 
 
 # ---------------------------------------------------------------- convolution / pooling
