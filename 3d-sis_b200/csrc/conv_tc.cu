@@ -41,7 +41,6 @@ struct TcArgs {
     int gemm_m, gemm_chunks_per_split;  // KS == 0 (plain GEMM y = x W^T, split-K over blockIdx.z)
     __half *out16;                      // optional fp16 twin of the output (same geometry as `out`); `out` may be null
     const float *bias_mid;              // N2 > 0: bias of the 3x3x3 conv (added before the inner ReLU), or null
-    int n_tiles;                        // bricks of this launch (the grid may be padded to a multiple of the cluster size)
 };
 
 __device__ __forceinline__ uint32_t smem_u32(const void *p) { return (uint32_t)__cvta_generic_to_shared(p); }
@@ -78,27 +77,6 @@ __device__ __forceinline__ void tma_load_2d(void *dst, const CUtensorMap *map, u
         ::"r"(smem_u32(dst)), "l"(reinterpret_cast<uint64_t>(map)), "r"(smem_u32(bar)), "r"(c0), "r"(c1)
         : "memory");
 }
-// cluster variants (CL = 2: two CTAs = two bricks of the same N tile share every weight tile: each CTA fetches half of them and
-// multicasts to both -> half the weight bytes per SM over the L2->SM crossbar, which bounds the wide / weight-heavy layers)
-__device__ __forceinline__ void tma_load_2d_mc(void *dst, const CUtensorMap *map, uint64_t *bar, int c0, int c1, uint16_t mask) {
-    asm volatile(
-        "cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes.multicast::cluster [%0], [%1, {%4, %5}], [%2], %3;"
-        ::"r"(smem_u32(dst)), "l"(reinterpret_cast<uint64_t>(map)), "r"(smem_u32(bar)), "h"(mask), "r"(c0), "r"(c1)
-        : "memory");
-}
-__device__ __forceinline__ void umma_commit_mc(uint64_t *bar, uint16_t mask) {
-    asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;"
-                 ::"r"(smem_u32(bar)), "h"(mask) : "memory");
-}
-__device__ __forceinline__ void cluster_sync_all() {
-    asm volatile("barrier.cluster.arrive.release.aligned;\n\tbarrier.cluster.wait.acquire.aligned;" ::: "memory");
-}
-__device__ __forceinline__ uint32_t cluster_ctarank() {
-    uint32_t r;
-    asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
-    return r;
-}
-
 // K-major, SWIZZLE_128B shared-memory matrix descriptor (cute::UMMA::SmemDescriptor bit layout):
 // start>>4 [0,14) | LBO=1 [16,30) | SBO=1024B>>4 [32,46) | version=1 [46,48) | layout=SWIZZLE_128B(2) [61,64)
 // ROWB = 128: SWIZZLE_128B (layout 2, 8-row atom = 1024 B);  ROWB = 64: SWIZZLE_64B (layout 4, 8-row atom = 512 B)
@@ -249,14 +227,13 @@ constexpr int tc_tmem_cols(int n) { return n <= 32 ? 32 : n <= 64 ? 64 : n <= 12
 // X3 = 2 (EB = 4, ROWB = 128): the same compensation with an fp16 split (split_f16 above): the fp32 slab lands in a staging
 // buffer, warps 2-3 write its hi and (scaled) lo parts as two fp16 K-major SWIZZLE_64B tiles, the weights are pre-split fp16
 // tiles, and the three products are kind::f16 MMAs -- same 22 significand bits, 2.5x the MMA rate, half as many stages.
-template <int BN, int KS, int EB = 4, int ROWB = 128, int BY = 2, int N2 = 0, int X3 = 0, int CL = 1>
+template <int BN, int KS, int EB = 4, int ROWB = 128, int BY = 2, int N2 = 0, int X3 = 0>
 __global__ void __launch_bounds__(X3 == 2 ? 256 : 128, (X3 == 2 && BN == 32) ? 2 : 1) conv3d_k3_tc_kernel(const __grid_constant__ CUtensorMap tmA,
                                                               const __grid_constant__ CUtensorMap tmB,
                                                               const __grid_constant__ CUtensorMap tmB2, const TcArgs a) {
     static_assert(N2 == 0 || (KS == 3 && EB == 4), "conv3 fusion: TF32 3x3x3 kernels only");
     static_assert(X3 == 0 || EB == 4, "3xTF32 splits fp32-stored operands");
     static_assert(X3 != 2 || ROWB == 128, "the fp16 split reads 128-byte fp32 rows and writes 64-byte fp16 rows");
-    static_assert(CL == 1 || (CL == 2 && KS == 3), "weight-tile multicast: pairs of 3x3x3 bricks");
     constexpr bool XH = X3 == 2;             // fp16 split
     // threads: warp 0 = TMA producer, warp 1 = MMA issuer, warps 2.. = operand splitters (X3), every warp = epilogue.  The fp16
     // split re-lays the slab out (fp32 128-byte rows -> two fp16 64-byte-row tiles), ~4 ALU ops per element: six splitter warps
@@ -304,7 +281,7 @@ __global__ void __launch_bounds__(X3 == 2 ? 256 : 128, (X3 == 2 && BN == 32) ? 2
 
     const int warp = threadIdx.x >> 5;
     if (threadIdx.x == 0) {
-        for (int i = 0; i < TC_STAGES; ++i) { mbar_init(full + i, 1); mbar_init(empty + i, CL); mbar_init(conv_done + i, NSPLIT); }
+        for (int i = 0; i < TC_STAGES; ++i) { mbar_init(full + i, 1); mbar_init(empty + i, 1); mbar_init(conv_done + i, NSPLIT); }
         mbar_init(acc_ready, 1);
         mbar_init(b2_full, 1);
         mbar_init(acc2_ready, 1);
@@ -319,21 +296,14 @@ __global__ void __launch_bounds__(X3 == 2 ? 256 : 128, (X3 == 2 && BN == 32) ? 2
     __syncthreads();
     asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
     const uint32_t tmem_base = *tmem_slot;
-    uint32_t crank = 0;
-    if constexpr (CL > 1) {
-        // both CTAs' barriers are initialised before either multicasts into the other's shared memory / arrives on its barriers
-        cluster_sync_all();
-        crank = cluster_ctarank();
-    }
 
     // ---- which brick
     int x0 = 0, y0 = 0, z0 = 0, x1 = 0, y1 = 0, z1 = 0;
     if constexpr (KS == 0) {
         // GEMM mode: rows instead of bricks (x0 = first row, set below)
     } else if (a.tiles) {
-        const int32_t *t = a.tiles + (size_t)min((int)blockIdx.x, a.n_tiles - 1) * 8;
+        const int32_t *t = a.tiles + (size_t)blockIdx.x * 8;
         x0 = t[0]; y0 = t[1]; z0 = t[2]; x1 = t[3]; y1 = t[4]; z1 = t[5];
-        if ((int)blockIdx.x >= a.n_tiles) x1 = y1 = z1 = 0;  // cluster padding: runs the pipeline (its peer needs it), stores nothing
     } else {
         const int tz = blockIdx.x % a.tiles_z, ty = (blockIdx.x / a.tiles_z) % a.tiles_y, tx = blockIdx.x / (a.tiles_z * a.tiles_y);
         x0 = tx * TC_BX; y0 = ty * TC_BY; z0 = tz * TC_BZ;
@@ -389,11 +359,7 @@ __global__ void __launch_bounds__(X3 == 2 ? 256 : 128, (X3 == 2 && BN == 32) ? 2
                     const int dx = j % 3, row0 = (j >= 3 ? a.cout : 0) + n0;
                     // weight columns k = ((dx*3+dy)*3+dz)*C_in + c  (X3 = 2: two halves per k -- [32 hi | 32 lo] per K slice)
                     const int kcol = (((dx * 3 + dy) * 3 + dz) * a.cin + kc * KC) * (XH ? 2 : 1);
-                    if constexpr (CL == 1) {
-                        tma_load_2d(sa + B_OFF + j * B_BYTES, &tmB, full + s, kcol, row0);
-                    } else if ((uint32_t)(j % CL) == crank) {  // this CTA's share of the pair's weight tiles, delivered to both
-                        tma_load_2d_mc(sa + B_OFF + j * B_BYTES, &tmB, full + s, kcol, row0, (uint16_t)((1u << CL) - 1u));
-                    }
+                    tma_load_2d(sa + B_OFF + j * B_BYTES, &tmB, full + s, kcol, row0);
                 }
             }
         }
@@ -436,9 +402,7 @@ __global__ void __launch_bounds__(X3 == 2 ? 256 : 128, (X3 == 2 && BN == 32) ? 2
                     else umma_f16(tmem_base, umma_desc<ROWB>(ax + k * 32), umma_desc<ROWB>(bx + k * 32), idesc, acc);
                 }
             }
-            // frees the smem slot once these MMAs retire (cluster: in BOTH CTAs -- the peer's producer multicasts into this slot too)
-            if constexpr (CL == 1) umma_commit(empty + s);
-            else umma_commit_mc(empty + s, (uint16_t)((1u << CL) - 1u));
+            umma_commit(empty + s);  // frees the smem slot once these MMAs retire
         }
         umma_commit(acc_ready);
     } else if (X3 && warp >= 2) {
@@ -647,7 +611,6 @@ __global__ void __launch_bounds__(X3 == 2 ? 256 : 128, (X3 == 2 && BN == 32) ? 2
     asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
     __syncthreads();
     if (warp == 1) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(TMEM_COLS) : "memory");
-    if constexpr (CL > 1) cluster_sync_all();  // no CTA exits while its peer may still multicast into it / arrive on its barriers
 }
 
 __global__ void gemm_splitk_reduce_kernel(const float *part, int splits, int64_t split_stride, const float *bias, float *y, int M,
@@ -703,49 +666,6 @@ __global__ void pack_conv_weight_tc_h3_kernel(const float *w, int cout, int cin,
     }
 }
 
-typedef CUresult (*EncodeTiledFn)(CUtensorMap *, CUtensorMapDataType, cuuint32_t, void *, const cuuint64_t *, const cuuint64_t *,
-                                  const cuuint32_t *, const cuuint32_t *, CUtensorMapInterleave, CUtensorMapSwizzle,
-                                  CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-static EncodeTiledFn get_encode() {
-    static EncodeTiledFn fn = nullptr;
-    if (!fn) {  // resolved through the runtime so libsis3d.so has no link-time dependency on libcuda
-        void *p = nullptr;
-        cudaDriverEntryPointQueryResult q;
-        if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) == cudaSuccess && q == cudaDriverEntryPointSuccess)
-            fn = (EncodeTiledFn)p;
-    }
-    return fn;
-}
-
-template <int BN, int KS, int EB = 4, int ROWB = 128, int BY = 2, int N2 = 0, int X3 = 0, int CL = 1>
-static int launch_tc(const CUtensorMap &tmA, const CUtensorMap &tmB, const TcArgs &a_in, int n_tiles, cudaStream_t s,
-                     const CUtensorMap *tmB2 = nullptr, int grid_z = 1) {
-    const size_t smem = tc_smem_bytes<BN, KS, ROWB, BY, N2, X3>();
-    auto kern = conv3d_k3_tc_kernel<BN, KS, EB, ROWB, BY, N2, X3, CL>;
-    static bool attr_done = false;
-    if (!attr_done) {
-        if (cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess)
-            return SIS3D_ELAUNCH;
-        attr_done = true;
-    }
-    TcArgs a = a_in;
-    a.n_tiles = n_tiles;
-    const int threads = X3 == 2 ? 256 : 128;
-    dim3 grid((n_tiles + CL - 1) / CL * CL, N2 > 0 ? 1 : a.cout / BN, grid_z);
-    if constexpr (CL == 1) {
-        kern<<<grid, threads, smem, s>>>(tmA, tmB, tmB2 ? *tmB2 : tmB, a);
-    } else {  // thread-block cluster of CL CTAs along x (pairs of bricks)
-        cudaLaunchConfig_t cfg = {};
-        cfg.gridDim = grid; cfg.blockDim = dim3(threads); cfg.dynamicSmemBytes = smem; cfg.stream = s;
-        cudaLaunchAttribute at[1];
-        at[0].id = cudaLaunchAttributeClusterDimension;
-        at[0].val.clusterDim.x = CL; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
-        cfg.attrs = at; cfg.numAttrs = 1;
-        if (cudaLaunchKernelEx(&cfg, kern, tmA, tmB, tmB2 ? *tmB2 : tmB, a) != cudaSuccess) return SIS3D_ELAUNCH;
-    }
-    return finish_launch();
-}
-
 // fp32 [cout][cin][taps] -> fp16 [cout][taps*cin] (k = tap*cin + c), round to nearest even
 __global__ void pack_conv_weight_tc_f16_kernel(const float *w, int cout, int cin, int taps, __half *out) {
     const int64_t total = (int64_t)cout * taps * cin;
@@ -771,280 +691,286 @@ __global__ void cast_f16_kernel(const float *in, int in_ld, int in_coff, int64_t
     }
 }
 
+typedef CUresult (*EncodeTiledFn)(CUtensorMap *, CUtensorMapDataType, cuuint32_t, void *, const cuuint64_t *, const cuuint64_t *,
+                                  const cuuint32_t *, const cuuint32_t *, CUtensorMapInterleave, CUtensorMapSwizzle,
+                                  CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
+static EncodeTiledFn get_encode() {
+    static EncodeTiledFn fn = nullptr;
+    if (!fn) {  // resolved through the runtime so libsis3d.so has no link-time dependency on libcuda
+        void *p = nullptr;
+        cudaDriverEntryPointQueryResult q;
+        if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) == cudaSuccess && q == cudaDriverEntryPointSuccess)
+            fn = (EncodeTiledFn)p;
+    }
+    return fn;
+}
+
+// ---- operand formats -------------------------------------------------------------------------------------------------------
+// One kernel serves four operand formats; a format fixes the kernel's EB / ROWB / X3, the element types of the two tensor maps
+// and the shape of the packed weight matrix.  Every box row is one swizzle span (128 or 64 bytes: SWIZZLE_128B / _64B).
+enum class TcFormat {
+    TF32,    // fp32 storage, kind::tf32
+    TF32X3,  // fp32 storage, split 3xTF32 (64-byte K rows so the hi and lo tiles fit the same shared memory)
+    F16X3,   // fp32 activations split in shared memory, pre-split fp16 weights, kind::f16
+    FP16,    // fp16 storage, kind::f16
+};
+struct TcFormatInfo {
+    int ab;                   // activation element bytes
+    int eb, rowb, x3;         // kernel template parameters EB, ROWB, X3
+    int wb;                   // weight element bytes (4: fp32, 2: fp16)
+    int kmul, nmul;           // packed weights are [cout * nmul][K * kmul]: f16x3 [32 hi | 32 lo] per 32-channel K slice,
+                              // tf32x3 hi rows then lo rows
+    int kc;                   // channels per pipeline stage (rowb / eb)
+    int bn_max;               // widest N tile
+};
+// fp16 storage: 64 channels per 128-byte row when cin allows it, else 32 per 64-byte row (C_in = 32), with N tiles of at most 64
+static TcFormatInfo tc_format(TcFormat f, int cin) {
+    switch (f) {
+        case TcFormat::TF32: return {4, 4, 128, 0, 4, 1, 1, 32, 128};
+        case TcFormat::TF32X3: return {4, 4, 64, 1, 4, 1, 2, 16, 128};
+        case TcFormat::F16X3: return {4, 4, 128, 2, 2, 2, 1, 32, 128};
+        default: return cin % 64 == 0 ? TcFormatInfo{2, 2, 128, 0, 2, 1, 1, 64, 128} : TcFormatInfo{2, 2, 64, 0, 2, 1, 1, 32, 64};
+    }
+}
+
+// ---- tensor maps -----------------------------------------------------------------------------------------------------------
+static CUtensorMapDataType tc_elem_type(int bytes) { return bytes == 4 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT32 : CU_TENSOR_MAP_DATA_TYPE_FLOAT16; }
+static CUtensorMapSwizzle tc_row_swizzle(int row_bytes) { return row_bytes == 128 ? CU_TENSOR_MAP_SWIZZLE_128B : CU_TENSOR_MAP_SWIZZLE_64B; }
+
+// A operand of the convolutions: the VC activation [X][Y][Z][cin], one box = kc channels of a (16/by) x by x 8 brick, plus a
+// one-plane x halo for ks = 3.  ks = 2 (stride 2, pad 0) traverses the input with element strides {1,2,2,2}; a box is given
+// in traversed elements, so N loaded voxels = box / stride.
+static bool encode_act(CUtensorMap *m, const TcFormatInfo &f, const void *in, int X, int Y, int Z, int cin, int ks, int by) {
+    const int sd = ks == 2 ? 2 : 1, bx = 16 / by;
+    cuuint64_t dims[4] = {(cuuint64_t)cin, (cuuint64_t)Z, (cuuint64_t)Y, (cuuint64_t)X};
+    cuuint64_t strides[3] = {(cuuint64_t)cin * f.ab, (cuuint64_t)Z * cin * f.ab, (cuuint64_t)Y * Z * cin * f.ab};
+    cuuint32_t box[4] = {(cuuint32_t)f.kc, (cuuint32_t)(TC_BZ * sd), (cuuint32_t)(by * sd), (cuuint32_t)((ks == 3 ? bx + 2 : bx) * sd)};
+    cuuint32_t estr[4] = {1, (cuuint32_t)sd, (cuuint32_t)sd, (cuuint32_t)sd};
+    return get_encode()(m, tc_elem_type(f.ab), 4, (void *)in, dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
+                        tc_row_swizzle(f.kc * f.ab), CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
+}
+// a row-major [rows][cols] matrix of eb-byte elements in boxes of box_rows x box_cols: packed weights (L2_256B promotion),
+// the fused tail's W3 and the GEMM's activations (L2_128B)
+static bool encode_mat(CUtensorMap *m, int eb, const void *p, int64_t cols, int64_t rows, int box_cols, int box_rows,
+                       CUtensorMapL2promotion l2) {
+    cuuint64_t dims[2] = {(cuuint64_t)cols, (cuuint64_t)rows};
+    cuuint64_t strides[1] = {(cuuint64_t)cols * eb};
+    cuuint32_t box[2] = {(cuuint32_t)box_cols, (cuuint32_t)box_rows};
+    cuuint32_t estr[2] = {1, 1};
+    return get_encode()(m, tc_elem_type(eb), 2, (void *)p, dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
+                        tc_row_swizzle(box_cols * eb), l2, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
+}
+constexpr CUtensorMapL2promotion kWeightL2 = CU_TENSOR_MAP_L2_PROMOTION_L2_256B;
+
+// ---- kernel variants -------------------------------------------------------------------------------------------------------
+template <int BN, int KS, int EB, int ROWB, int BY, int N2, int X3>
+static int launch_tc(const CUtensorMap &tmA, const CUtensorMap &tmB, const CUtensorMap &tmB2, const TcArgs &a, int n_tiles,
+                     int grid_z, cudaStream_t s) {
+    const size_t smem = tc_smem_bytes<BN, KS, ROWB, BY, N2, X3>();
+    auto kern = conv3d_k3_tc_kernel<BN, KS, EB, ROWB, BY, N2, X3>;
+    static bool attr_done = false;
+    if (!attr_done) {
+        if (cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess)
+            return SIS3D_ELAUNCH;
+        attr_done = true;
+    }
+    kern<<<dim3(n_tiles, N2 > 0 ? 1 : a.cout / BN, grid_z), X3 == 2 ? 256 : 128, smem, s>>>(tmA, tmB, tmB2, a);
+    return finish_launch();
+}
+
+struct TcVariant {
+    int bn, ks, eb, rowb, by, n2, x3;
+    int (*launch)(const CUtensorMap &, const CUtensorMap &, const CUtensorMap &, const TcArgs &, int, int, cudaStream_t);
+};
+#define TC_VARIANT(BN, KS, EB, ROWB, BY, N2, X3) {BN, KS, EB, ROWB, BY, N2, X3, launch_tc<BN, KS, EB, ROWB, BY, N2, X3>}
+// Every instantiation of conv3d_k3_tc_kernel.  KS = 0 is the GEMM; N2 > 0 the fused bottleneck tail (BN = cmid, N2 = cout);
+// BY = 4 the 4x4x8 bricks of tile lists with cout = 64.
+static const TcVariant kTcVariants[] = {
+    // tf32
+    TC_VARIANT(32, 3, 4, 128, 2, 0, 0), TC_VARIANT(64, 3, 4, 128, 2, 0, 0), TC_VARIANT(128, 3, 4, 128, 2, 0, 0),
+    TC_VARIANT(64, 3, 4, 128, 4, 0, 0),
+    TC_VARIANT(32, 2, 4, 128, 2, 0, 0), TC_VARIANT(64, 2, 4, 128, 2, 0, 0), TC_VARIANT(128, 2, 4, 128, 2, 0, 0),
+    TC_VARIANT(32, 1, 4, 128, 2, 0, 0), TC_VARIANT(64, 1, 4, 128, 2, 0, 0), TC_VARIANT(128, 1, 4, 128, 2, 0, 0),
+    TC_VARIANT(32, 0, 4, 128, 2, 0, 0), TC_VARIANT(64, 0, 4, 128, 2, 0, 0), TC_VARIANT(128, 0, 4, 128, 2, 0, 0),
+    TC_VARIANT(32, 3, 4, 128, 2, 32, 0), TC_VARIANT(32, 3, 4, 128, 2, 64, 0), TC_VARIANT(64, 3, 4, 128, 2, 128, 0),
+    // tf32x3
+    TC_VARIANT(32, 3, 4, 64, 2, 0, 1), TC_VARIANT(64, 3, 4, 64, 2, 0, 1), TC_VARIANT(128, 3, 4, 64, 2, 0, 1),
+    TC_VARIANT(32, 2, 4, 64, 2, 0, 1), TC_VARIANT(64, 2, 4, 64, 2, 0, 1), TC_VARIANT(128, 2, 4, 64, 2, 0, 1),
+    TC_VARIANT(32, 1, 4, 64, 2, 0, 1), TC_VARIANT(64, 1, 4, 64, 2, 0, 1), TC_VARIANT(128, 1, 4, 64, 2, 0, 1),
+    TC_VARIANT(32, 0, 4, 64, 2, 0, 1), TC_VARIANT(64, 0, 4, 64, 2, 0, 1), TC_VARIANT(128, 0, 4, 64, 2, 0, 1),
+    TC_VARIANT(32, 3, 4, 64, 2, 32, 1), TC_VARIANT(32, 3, 4, 64, 2, 64, 1), TC_VARIANT(64, 3, 4, 64, 2, 128, 1),
+    // f16x3
+    TC_VARIANT(32, 3, 4, 128, 2, 0, 2), TC_VARIANT(64, 3, 4, 128, 2, 0, 2), TC_VARIANT(128, 3, 4, 128, 2, 0, 2),
+    TC_VARIANT(32, 2, 4, 128, 2, 0, 2), TC_VARIANT(64, 2, 4, 128, 2, 0, 2), TC_VARIANT(128, 2, 4, 128, 2, 0, 2),
+    TC_VARIANT(32, 1, 4, 128, 2, 0, 2), TC_VARIANT(64, 1, 4, 128, 2, 0, 2), TC_VARIANT(128, 1, 4, 128, 2, 0, 2),
+    TC_VARIANT(32, 0, 4, 128, 2, 0, 2), TC_VARIANT(64, 0, 4, 128, 2, 0, 2), TC_VARIANT(128, 0, 4, 128, 2, 0, 2),
+    TC_VARIANT(32, 3, 4, 128, 2, 32, 2), TC_VARIANT(32, 3, 4, 128, 2, 64, 2), TC_VARIANT(64, 3, 4, 128, 2, 128, 2),
+    // fp16, 128-byte rows
+    TC_VARIANT(32, 3, 2, 128, 2, 0, 0), TC_VARIANT(64, 3, 2, 128, 2, 0, 0), TC_VARIANT(128, 3, 2, 128, 2, 0, 0),
+    TC_VARIANT(64, 3, 2, 128, 4, 0, 0),
+    TC_VARIANT(32, 1, 2, 128, 2, 0, 0), TC_VARIANT(64, 1, 2, 128, 2, 0, 0), TC_VARIANT(128, 1, 2, 128, 2, 0, 0),
+    // fp16, 64-byte rows
+    TC_VARIANT(32, 3, 2, 64, 2, 0, 0), TC_VARIANT(64, 3, 2, 64, 2, 0, 0),
+    TC_VARIANT(32, 1, 2, 64, 2, 0, 0), TC_VARIANT(64, 1, 2, 64, 2, 0, 0),
+};
+#undef TC_VARIANT
+static const TcVariant *tc_variant(const TcFormatInfo &f, int ks, int bn, int by, int n2) {
+    for (const TcVariant &v : kTcVariants)
+        if (v.eb == f.eb && v.rowb == f.rowb && v.x3 == f.x3 && v.ks == ks && v.bn == bn && v.by == by && v.n2 == n2) return &v;
+    return nullptr;
+}
+
+// brick height: explicit tile lists (ragged RoI crops) of 64 -> 64 3x3x3 layers use 4x4x8 bricks, everything else 8x2x8
+static int tc_brick_y(bool with_tile_list, int ks, int cin, int cout) {
+    return (with_tile_list && ks == 3 && cout == 64 && cin % 64 == 0) ? 4 : 2;
+}
+
 }  // namespace sis3d
 using namespace sis3d;
 
-extern "C" int sis3d_pack_conv_weight_tc(const float *w, int cout, int cin, int ks, float *w_tc, void *stream) {
-    if (!w || !w_tc || cout <= 0 || cin <= 0 || (ks != 1 && ks != 2 && ks != 3)) return SIS3D_EINVAL;
+template <typename T>
+static int pack_tc(void (*kern)(const float *, int, int, int, T *), const float *w, int cout, int cin, int ks, T *out, void *stream) {
+    if (!w || !out || cout <= 0 || cin <= 0 || (ks != 1 && ks != 2 && ks != 3)) return SIS3D_EINVAL;
     const int taps = ks * ks * ks;
     const int64_t total = (int64_t)cout * taps * cin;
-    pack_conv_weight_tc_kernel<<<(int)imin64(cdiv64(total, 256), 148 * 8), 256, 0, (cudaStream_t)stream>>>(w, cout, cin, taps, w_tc);
+    kern<<<(int)imin64(cdiv64(total, 256), 148 * 8), 256, 0, (cudaStream_t)stream>>>(w, cout, cin, taps, out);
     return finish_launch();
+}
+extern "C" int sis3d_pack_conv_weight_tc(const float *w, int cout, int cin, int ks, float *w_tc, void *stream) {
+    return pack_tc(pack_conv_weight_tc_kernel, w, cout, cin, ks, w_tc, stream);
+}
+extern "C" int sis3d_pack_conv_weight_tc_x3(const float *w, int cout, int cin, int ks, float *w_x3, void *stream) {
+    return pack_tc(pack_conv_weight_tc_x3_kernel, w, cout, cin, ks, w_x3, stream);
+}
+extern "C" int sis3d_pack_conv_weight_tc_h3(const float *w, int cout, int cin, int ks, uint16_t *w_h3, void *stream) {
+    return pack_tc(pack_conv_weight_tc_h3_kernel, w, cout, cin, ks, (__half *)w_h3, stream);
+}
+extern "C" int sis3d_pack_conv_weight_tc_f16(const float *w, int cout, int cin, int ks, uint16_t *w16, void *stream) {
+    if (ks == 2) return SIS3D_EINVAL;  // fp16 storage has no 2x2x2 kernel
+    return pack_tc(pack_conv_weight_tc_f16_kernel, w, cout, cin, ks, (__half *)w16, stream);
 }
 
 extern "C" int sis3d_conv3d_k3_tc_supported(int cin, int cout) {
     return (cin % TC_KC == 0 && (cout == 32 || cout == 64 || cout % 128 == 0)) ? 1 : 0;
 }
 
-extern "C" int sis3d_pack_conv_weight_tc_x3(const float *w, int cout, int cin, int ks, float *w_x3, void *stream) {
-    if (!w || !w_x3 || cout <= 0 || cin <= 0 || (ks != 1 && ks != 2 && ks != 3)) return SIS3D_EINVAL;
-    const int taps = ks * ks * ks;
-    const int64_t total = (int64_t)cout * taps * cin;
-    pack_conv_weight_tc_x3_kernel<<<(int)imin64(cdiv64(total, 256), 148 * 8), 256, 0, (cudaStream_t)stream>>>(w, cout, cin, taps, w_x3);
-    return finish_launch();
-}
-
-extern "C" int sis3d_pack_conv_weight_tc_h3(const float *w, int cout, int cin, int ks, uint16_t *w_h3, void *stream) {
-    if (!w || !w_h3 || cout <= 0 || cin <= 0 || (ks != 1 && ks != 2 && ks != 3)) return SIS3D_EINVAL;
-    const int taps = ks * ks * ks;
-    const int64_t total = (int64_t)cout * taps * cin;
-    pack_conv_weight_tc_h3_kernel<<<(int)imin64(cdiv64(total, 256), 148 * 8), 256, 0, (cudaStream_t)stream>>>(w, cout, cin, taps, (__half *)w_h3);
-    return finish_launch();
-}
-
-// SIS3D_CLUSTER=1 turns the 2-CTA weight-tile multicast ON (validated: all parity tests pass with it; measured on B200 it does not
-// pay -- 2414 vs 2529 scenes/s, rpn_net 44.5 vs 44.0 us -- because the bound is the rate at which an SM RECEIVES TMA rows, which
-// multicast does not change; kept as an A/B switch)
-static bool use_cluster() {
-    static const bool on = getenv("SIS3D_CLUSTER") != nullptr && getenv("SIS3D_CLUSTER")[0] == '1';
-    return on;
-}
-
-static int conv3d_k3_tc_impl(const float *in, const float *w_tc, const float *bias, const float *residual, int res_ld,
-                             int res_coff, float *out, int out_ld, int out_coff, int X, int Y, int Z, int cin, int cout,
-                             int ks, const int32_t *tiles, int n_tiles, int act, void *stream, int x3) {
-    if (!in || !w_tc || !out || X <= 0 || Y <= 0 || Z <= 0 || (ks != 1 && ks != 2 && ks != 3)) return SIS3D_EINVAL;
+// One convolution in any format.  out16 (an fp16 twin of the output, `out` may then be null) exists only with fp16 storage, which
+// has no 2x2x2 kernel; the compensated formats take whole volumes only.
+static int conv_tc(TcFormat fmt, const void *in, const void *w, const float *bias, const float *residual, int res_ld, int res_coff,
+                   float *out, uint16_t *out16, int out_ld, int out_coff, int X, int Y, int Z, int cin, int cout, int ks,
+                   const int32_t *tiles, int n_tiles, int act, void *stream) {
+    const bool ks_ok = ks == 1 || ks == 3 || (ks == 2 && fmt != TcFormat::FP16);
+    if (!in || !w || (!out && !out16) || X <= 0 || Y <= 0 || Z <= 0 || !ks_ok) return SIS3D_EINVAL;
     if (ks == 2 && (tiles || X < 2 || Y < 2 || Z < 2)) return SIS3D_EINVAL;
-    if (x3 && tiles) return SIS3D_EUNSUPPORTED;  // the ragged mask stage does not need the compensated product
-    const int taps = ks * ks * ks;
-    // explicit tile lists (ragged RoI crops) use 4x4x8 bricks, whole volumes 8x2x8 (sis3d_conv3d_tc_brick)
-    const int by = (tiles && ks == 3 && cout == 64 && cin % 64 == 0) ? 4 : 2, bx = 16 / by;
+    const TcFormatInfo f = tc_format(fmt, cin);
+    if (f.x3 && tiles) return SIS3D_EUNSUPPORTED;  // the ragged mask stage does not need the compensated product
     if (!sis3d_conv3d_k3_tc_supported(cin, cout)) return SIS3D_EUNSUPPORTED;
-    if (((uintptr_t)in | (uintptr_t)w_tc | (uintptr_t)out) & 15) return SIS3D_EINVAL;
+    if (((uintptr_t)in | (uintptr_t)w | (uintptr_t)out | (uintptr_t)out16) & 15) return SIS3D_EINVAL;
     if ((out_ld | out_coff | res_ld | res_coff) & 3) return SIS3D_EINVAL;
-    EncodeTiledFn enc = get_encode();
-    if (!enc) return SIS3D_EUNSUPPORTED;
-    const int BN = cout >= 128 ? 128 : cout;
-    // x3 = 1 (TF32 split): 64-byte K rows (SWIZZLE_64B) so hi + lo tiles fit the same smem; x3 = 2 (fp16 split): 128-byte fp32
-    // activation rows, pre-split fp16 weights in 64-byte rows
-    const int kc = x3 == 1 ? 16 : TC_KC;
-    const CUtensorMapSwizzle sw = x3 == 1 ? CU_TENSOR_MAP_SWIZZLE_64B : CU_TENSOR_MAP_SWIZZLE_128B;
-    const CUtensorMapSwizzle swb = x3 == 1 ? CU_TENSOR_MAP_SWIZZLE_64B : CU_TENSOR_MAP_SWIZZLE_128B;
-    const CUtensorMapDataType dtb = x3 == 2 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT32;
-    const cuuint64_t wb = x3 == 2 ? 2 : 4;  // weight element bytes
+    if (!get_encode()) return SIS3D_EUNSUPPORTED;
+    if (fmt == TcFormat::FP16 && cin % 64 != 0 && cin != 32) return SIS3D_EUNSUPPORTED;
+    const int by = tc_brick_y(tiles != nullptr, ks, cin, cout), bx = 16 / by;
+    const int BN = min(cout, f.bn_max);
     const int sd = ks == 2 ? 2 : 1;                   // ks == 2 is the stride-2, pad-0 conv: X, Y, Z are the INPUT extents
     const int Xo = X / sd, Yo = Y / sd, Zo = Z / sd;  // output extents (floor, as nn.Conv3d)
     CUtensorMap tmA, tmB;
-    {
-        cuuint64_t dims[4] = {(cuuint64_t)cin, (cuuint64_t)Z, (cuuint64_t)Y, (cuuint64_t)X};
-        cuuint64_t strides[3] = {(cuuint64_t)cin * 4, (cuuint64_t)Z * cin * 4, (cuuint64_t)Y * Z * cin * 4};
-        // with element strides the box is given in traversed elements: N loaded voxels = boxDim / stride
-        cuuint32_t box[4] = {(cuuint32_t)kc, (cuuint32_t)(TC_BZ * sd), (cuuint32_t)(by * sd), (cuuint32_t)((ks == 3 ? bx + 2 : bx) * sd)};
-        cuuint32_t estr[4] = {1, (cuuint32_t)sd, (cuuint32_t)sd, (cuuint32_t)sd};
-        if (enc(&tmA, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, (void *)in, dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                sw, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) != CUDA_SUCCESS)
-            return SIS3D_EINVAL;
-    }
-    {
-        // x3 = 1: hi rows, then lo rows; x3 = 2: [32 hi | 32 lo] halves per 32-channel K slice in one 128-byte row
-        cuuint64_t dims[2] = {(cuuint64_t)taps * cin * (x3 == 2 ? 2 : 1), (cuuint64_t)cout * (x3 == 1 ? 2 : 1)};
-        cuuint64_t strides[1] = {dims[0] * wb};
-        cuuint32_t box[2] = {(cuuint32_t)(x3 == 2 ? 64 : kc), (cuuint32_t)BN};
-        cuuint32_t estr[2] = {1, 1};
-        if (enc(&tmB, dtb, 2, (void *)w_tc, dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                swb, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) != CUDA_SUCCESS)
-            return SIS3D_EINVAL;
-    }
-    TcArgs a;
-    a.bias = bias; a.res = residual; a.out = out; a.tiles = tiles; a.out16 = nullptr; a.bias_mid = nullptr;
+    if (!encode_act(&tmA, f, in, X, Y, Z, cin, ks, by) ||
+        !encode_mat(&tmB, f.wb, w, (int64_t)ks * ks * ks * cin * f.kmul, (int64_t)cout * f.nmul, f.kc * f.kmul, BN, kWeightL2))
+        return SIS3D_EINVAL;
+    TcArgs a = {};
+    a.bias = bias; a.res = residual; a.out = out; a.out16 = (__half *)out16; a.tiles = tiles;
     a.X = Xo; a.Y = Yo; a.Z = Zo; a.cin = cin; a.cout = cout; a.act = act;
     a.out_ld = out_ld; a.out_coff = out_coff; a.res_ld = res_ld; a.res_coff = res_coff;
     a.tiles_y = cdiv(Yo, by); a.tiles_z = cdiv(Zo, TC_BZ);
     if (!tiles) n_tiles = cdiv(Xo, bx) * a.tiles_y * a.tiles_z;
     if (n_tiles <= 0) return SIS3D_OK;
-    cudaStream_t s = (cudaStream_t)stream;
-    if (x3 == 2) {
-        if (ks == 3) {
-            switch (BN) {
-                case 32: return launch_tc<32, 3, 4, 128, 2, 0, 2>(tmA, tmB, a, n_tiles, s);
-                case 64: return launch_tc<64, 3, 4, 128, 2, 0, 2>(tmA, tmB, a, n_tiles, s);
-                default: return use_cluster() ? launch_tc<128, 3, 4, 128, 2, 0, 2, 2>(tmA, tmB, a, n_tiles, s)
-                                              : launch_tc<128, 3, 4, 128, 2, 0, 2>(tmA, tmB, a, n_tiles, s);
-            }
-        }
-        if (ks == 2) {
-            switch (BN) {
-                case 32: return launch_tc<32, 2, 4, 128, 2, 0, 2>(tmA, tmB, a, n_tiles, s);
-                case 64: return launch_tc<64, 2, 4, 128, 2, 0, 2>(tmA, tmB, a, n_tiles, s);
-                default: return launch_tc<128, 2, 4, 128, 2, 0, 2>(tmA, tmB, a, n_tiles, s);
-            }
-        }
-        switch (BN) {
-            case 32: return launch_tc<32, 1, 4, 128, 2, 0, 2>(tmA, tmB, a, n_tiles, s);
-            case 64: return launch_tc<64, 1, 4, 128, 2, 0, 2>(tmA, tmB, a, n_tiles, s);
-            default: return launch_tc<128, 1, 4, 128, 2, 0, 2>(tmA, tmB, a, n_tiles, s);
-        }
-    }
-    if (x3) {
-        if (ks == 3) {
-            switch (BN) {
-                case 32: return launch_tc<32, 3, 4, 64, 2, 0, 1>(tmA, tmB, a, n_tiles, s);
-                case 64: return launch_tc<64, 3, 4, 64, 2, 0, 1>(tmA, tmB, a, n_tiles, s);
-                default: return launch_tc<128, 3, 4, 64, 2, 0, 1>(tmA, tmB, a, n_tiles, s);
-            }
-        }
-        if (ks == 2) {
-            switch (BN) {
-                case 32: return launch_tc<32, 2, 4, 64, 2, 0, 1>(tmA, tmB, a, n_tiles, s);
-                case 64: return launch_tc<64, 2, 4, 64, 2, 0, 1>(tmA, tmB, a, n_tiles, s);
-                default: return launch_tc<128, 2, 4, 64, 2, 0, 1>(tmA, tmB, a, n_tiles, s);
-            }
-        }
-        switch (BN) {
-            case 32: return launch_tc<32, 1, 4, 64, 2, 0, 1>(tmA, tmB, a, n_tiles, s);
-            case 64: return launch_tc<64, 1, 4, 64, 2, 0, 1>(tmA, tmB, a, n_tiles, s);
-            default: return launch_tc<128, 1, 4, 64, 2, 0, 1>(tmA, tmB, a, n_tiles, s);
-        }
-    }
-    if (ks == 3) {
-        if (by == 4) return use_cluster() ? launch_tc<64, 3, 4, 128, 4, 0, 0, 2>(tmA, tmB, a, n_tiles, s)
-                                          : launch_tc<64, 3, 4, 128, 4>(tmA, tmB, a, n_tiles, s);
-        switch (BN) {
-            case 32: return launch_tc<32, 3>(tmA, tmB, a, n_tiles, s);
-            case 64: return launch_tc<64, 3>(tmA, tmB, a, n_tiles, s);
-            default: return launch_tc<128, 3>(tmA, tmB, a, n_tiles, s);
-        }
-    }
-    if (ks == 2) {
-        switch (BN) {
-            case 32: return launch_tc<32, 2>(tmA, tmB, a, n_tiles, s);
-            case 64: return launch_tc<64, 2>(tmA, tmB, a, n_tiles, s);
-            default: return launch_tc<128, 2>(tmA, tmB, a, n_tiles, s);
-        }
-    }
-    switch (BN) {
-        case 32: return launch_tc<32, 1>(tmA, tmB, a, n_tiles, s);
-        case 64: return launch_tc<64, 1>(tmA, tmB, a, n_tiles, s);
-        default: return launch_tc<128, 1>(tmA, tmB, a, n_tiles, s);
-    }
+    const TcVariant *v = tc_variant(f, ks, BN, by, 0);
+    return v ? v->launch(tmA, tmB, tmB, a, n_tiles, 1, (cudaStream_t)stream) : SIS3D_EUNSUPPORTED;
 }
 extern "C" int sis3d_conv3d_k3_tc(const float *in, const float *w_tc, const float *bias, const float *residual, int res_ld,
                                   int res_coff, float *out, int out_ld, int out_coff, int X, int Y, int Z, int cin, int cout,
                                   int ks, const int32_t *tiles, int n_tiles, int act, void *stream) {
-    return conv3d_k3_tc_impl(in, w_tc, bias, residual, res_ld, res_coff, out, out_ld, out_coff, X, Y, Z, cin, cout, ks, tiles,
-                             n_tiles, act, stream, 0);
+    return conv_tc(TcFormat::TF32, in, w_tc, bias, residual, res_ld, res_coff, out, nullptr, out_ld, out_coff, X, Y, Z, cin, cout, ks,
+                   tiles, n_tiles, act, stream);
 }
 // error-compensated 3xTF32 (fp32-class accuracy on the tensor cores): w_x3 from sis3d_pack_conv_weight_tc_x3
 extern "C" int sis3d_conv3d_k3_tc_x3(const float *in, const float *w_x3, const float *bias, const float *residual, int res_ld,
                                      int res_coff, float *out, int out_ld, int out_coff, int X, int Y, int Z, int cin, int cout,
                                      int ks, int act, void *stream) {
-    return conv3d_k3_tc_impl(in, w_x3, bias, residual, res_ld, res_coff, out, out_ld, out_coff, X, Y, Z, cin, cout, ks, nullptr, 0,
-                             act, stream, 1);
+    return conv_tc(TcFormat::TF32X3, in, w_x3, bias, residual, res_ld, res_coff, out, nullptr, out_ld, out_coff, X, Y, Z, cin, cout,
+                   ks, nullptr, 0, act, stream);
 }
 // the same compensation with an fp16 operand split (2.5x the MMA rate): w_h3 from sis3d_pack_conv_weight_tc_h3
 extern "C" int sis3d_conv3d_k3_tc_h3(const float *in, const uint16_t *w_h3, const float *bias, const float *residual, int res_ld,
                                      int res_coff, float *out, int out_ld, int out_coff, int X, int Y, int Z, int cin, int cout,
                                      int ks, int act, void *stream) {
-    return conv3d_k3_tc_impl(in, (const float *)w_h3, bias, residual, res_ld, res_coff, out, out_ld, out_coff, X, Y, Z, cin, cout,
-                             ks, nullptr, 0, act, stream, 2);
+    return conv_tc(TcFormat::F16X3, in, w_h3, bias, residual, res_ld, res_coff, out, nullptr, out_ld, out_coff, X, Y, Z, cin, cout,
+                   ks, nullptr, 0, act, stream);
+}
+// fp16-operand variant (kind::f16): activations and weights stored as fp16, fp32 accumulation in TMEM
+extern "C" int sis3d_conv3d_tc_f16(const uint16_t *in16, const uint16_t *w16, const float *bias, const float *residual,
+                                   int res_ld, int res_coff, float *out32, uint16_t *out16, int out_ld, int out_coff, int X, int Y,
+                                   int Z, int cin, int cout, int ks, const int32_t *tiles, int n_tiles, int act, void *stream) {
+    return conv_tc(TcFormat::FP16, in16, w16, bias, residual, res_ld, res_coff, out32, out16, out_ld, out_coff, X, Y, Z, cin, cout, ks,
+                   tiles, n_tiles, act, stream);
+}
+extern "C" int sis3d_cast_f16(const float *in, int in_ld, int in_coff, int64_t rows, int C, uint16_t *out, void *stream) {
+    if (!in || !out || rows <= 0 || C % 4 != 0 || (in_ld | in_coff) & 3) return SIS3D_EINVAL;
+    cast_f16_kernel<<<(int)imin64(cdiv64(rows * (C / 4), 256), 148 * 8), 256, 0, (cudaStream_t)stream>>>(in, in_ld, in_coff, rows, C / 4, (__half *)out);
+    return finish_launch();
 }
 
 // ---- bottleneck tail: 3x3x3 conv (cin -> cmid) + ReLU + 1x1 conv (cmid -> cout) + residual + act, one kernel ----------------
 extern "C" int sis3d_conv3d_k3_tc_fused_supported(int cin, int cmid, int cout) {
     return (cin % TC_KC == 0 && ((cmid == 32 && (cout == 32 || cout == 64)) || (cmid == 64 && cout == 128))) ? 1 : 0;
 }
-static int conv3d_k3_tc_fused_impl(const float *in, const float *w2_tc, const float *bias2, const float *w3_tc,
-                                   const float *bias3, const float *residual, int res_ld, int res_coff, float *out,
-                                   int out_ld, int out_coff, int X, int Y, int Z, int cin, int cmid, int cout, int act,
-                                   void *stream, int x3) {
-    if (!in || !w2_tc || !w3_tc || !out || X <= 0 || Y <= 0 || Z <= 0) return SIS3D_EINVAL;
+static int conv_tc_fused(TcFormat fmt, const float *in, const void *w2, const float *bias2, const void *w3, const float *bias3,
+                         const float *residual, int res_ld, int res_coff, float *out, int out_ld, int out_coff, int X, int Y, int Z,
+                         int cin, int cmid, int cout, int act, void *stream) {
+    if (!in || !w2 || !w3 || !out || X <= 0 || Y <= 0 || Z <= 0) return SIS3D_EINVAL;
     if (!sis3d_conv3d_k3_tc_fused_supported(cin, cmid, cout)) return SIS3D_EUNSUPPORTED;
-    if (((uintptr_t)in | (uintptr_t)w2_tc | (uintptr_t)w3_tc | (uintptr_t)out) & 15) return SIS3D_EINVAL;
+    if (((uintptr_t)in | (uintptr_t)w2 | (uintptr_t)w3 | (uintptr_t)out) & 15) return SIS3D_EINVAL;
     if ((out_ld | out_coff | res_ld | res_coff) & 3) return SIS3D_EINVAL;
-    EncodeTiledFn enc = get_encode();
-    if (!enc) return SIS3D_EUNSUPPORTED;
-    const int by = 2, bx = 8;
-    const int kc = x3 == 1 ? 16 : TC_KC;
-    const CUtensorMapSwizzle sw = x3 == 1 ? CU_TENSOR_MAP_SWIZZLE_64B : CU_TENSOR_MAP_SWIZZLE_128B;
-    const CUtensorMapSwizzle swb = x3 == 1 ? CU_TENSOR_MAP_SWIZZLE_64B : CU_TENSOR_MAP_SWIZZLE_128B;
-    const CUtensorMapSwizzle swb2 = CU_TENSOR_MAP_SWIZZLE_128B;
-    const CUtensorMapDataType dtb = x3 == 2 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT32;
-    const cuuint64_t wb = x3 == 2 ? 2 : 4;
-    const int halves = x3 == 1 ? 2 : 1;  // x3 = 1 weight tensors: hi rows, then lo rows
-    const int kmul = x3 == 2 ? 2 : 1;    // x3 = 2: [32 hi | 32 lo] halves per K slice in one row
+    if (!get_encode()) return SIS3D_EUNSUPPORTED;
+    const TcFormatInfo f = tc_format(fmt, cin);
     CUtensorMap tmA, tmB, tmB2;
-    cuuint32_t estr[4] = {1, 1, 1, 1};
-    {
-        cuuint64_t dims[4] = {(cuuint64_t)cin, (cuuint64_t)Z, (cuuint64_t)Y, (cuuint64_t)X};
-        cuuint64_t strides[3] = {(cuuint64_t)cin * 4, (cuuint64_t)Z * cin * 4, (cuuint64_t)Y * Z * cin * 4};
-        cuuint32_t box[4] = {(cuuint32_t)kc, TC_BZ, (cuuint32_t)by, (cuuint32_t)(bx + 2)};
-        if (enc(&tmA, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, (void *)in, dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                sw, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) != CUDA_SUCCESS)
-            return SIS3D_EINVAL;
-    }
-    {
-        cuuint64_t dims[2] = {(cuuint64_t)27 * cin * kmul, (cuuint64_t)cmid * halves};
-        cuuint64_t strides[1] = {dims[0] * wb};
-        cuuint32_t box[2] = {(cuuint32_t)(x3 == 2 ? 64 : kc), (cuuint32_t)cmid};
-        if (enc(&tmB, dtb, 2, (void *)w2_tc, dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                swb, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) != CUDA_SUCCESS)
-            return SIS3D_EINVAL;
-    }
-    {
-        cuuint64_t dims[2] = {(cuuint64_t)cmid * kmul, (cuuint64_t)cout * halves};
-        cuuint64_t strides[1] = {dims[0] * wb};
-        cuuint32_t box[2] = {(cuuint32_t)(TC_KC * kmul), (cuuint32_t)cout};
-        if (enc(&tmB2, dtb, 2, (void *)w3_tc, dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                swb2, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) != CUDA_SUCCESS)
-            return SIS3D_EINVAL;
-    }
-    TcArgs a;
-    a.bias = bias3; a.bias_mid = bias2; a.res = residual; a.out = out; a.tiles = nullptr; a.out16 = nullptr;
+    if (!encode_act(&tmA, f, in, X, Y, Z, cin, 3, 2) ||
+        !encode_mat(&tmB, f.wb, w2, (int64_t)27 * cin * f.kmul, (int64_t)cmid * f.nmul, f.kc * f.kmul, cmid, kWeightL2) ||
+        !encode_mat(&tmB2, f.wb, w3, (int64_t)cmid * f.kmul, (int64_t)cout * f.nmul, TC_KC * f.kmul, cout, kWeightL2))
+        return SIS3D_EINVAL;
+    TcArgs a = {};
+    a.bias = bias3; a.bias_mid = bias2; a.res = residual; a.out = out;
     // the main loop's weight rows (and their lo halves, x3) are indexed with the 3x3x3 conv's width, the epilogue with cout
-    a.X = X; a.Y = Y; a.Z = Z; a.cin = cin; a.cout = x3 ? cmid : cout; a.act = act;
+    a.X = X; a.Y = Y; a.Z = Z; a.cin = cin; a.cout = f.x3 ? cmid : cout; a.act = act;
     a.out_ld = out_ld; a.out_coff = out_coff; a.res_ld = res_ld; a.res_coff = res_coff;
-    a.tiles_y = cdiv(Y, by); a.tiles_z = cdiv(Z, TC_BZ);
-    a.gemm_m = 0; a.gemm_chunks_per_split = 0;
-    const int n_tiles = cdiv(X, bx) * a.tiles_y * a.tiles_z;
-    cudaStream_t s = (cudaStream_t)stream;
-    if (x3 == 2) {
-        if (cmid == 32 && cout == 32) return launch_tc<32, 3, 4, 128, 2, 32, 2>(tmA, tmB, a, n_tiles, s, &tmB2);
-        if (cmid == 32 && cout == 64) return launch_tc<32, 3, 4, 128, 2, 64, 2>(tmA, tmB, a, n_tiles, s, &tmB2);
-        return use_cluster() ? launch_tc<64, 3, 4, 128, 2, 128, 2, 2>(tmA, tmB, a, n_tiles, s, &tmB2)
-                             : launch_tc<64, 3, 4, 128, 2, 128, 2>(tmA, tmB, a, n_tiles, s, &tmB2);
-    }
-    if (x3) {
-        if (cmid == 32 && cout == 32) return launch_tc<32, 3, 4, 64, 2, 32, 1>(tmA, tmB, a, n_tiles, s, &tmB2);
-        if (cmid == 32 && cout == 64) return launch_tc<32, 3, 4, 64, 2, 64, 1>(tmA, tmB, a, n_tiles, s, &tmB2);
-        return launch_tc<64, 3, 4, 64, 2, 128, 1>(tmA, tmB, a, n_tiles, s, &tmB2);
-    }
-    if (cmid == 32 && cout == 32) return launch_tc<32, 3, 4, 128, 2, 32>(tmA, tmB, a, n_tiles, s, &tmB2);
-    if (cmid == 32 && cout == 64) return launch_tc<32, 3, 4, 128, 2, 64>(tmA, tmB, a, n_tiles, s, &tmB2);
-    return launch_tc<64, 3, 4, 128, 2, 128>(tmA, tmB, a, n_tiles, s, &tmB2);
+    a.tiles_y = cdiv(Y, 2); a.tiles_z = cdiv(Z, TC_BZ);
+    const int n_tiles = cdiv(X, 8) * a.tiles_y * a.tiles_z;
+    const TcVariant *v = tc_variant(f, 3, cmid, 2, cout);
+    return v ? v->launch(tmA, tmB, tmB2, a, n_tiles, 1, (cudaStream_t)stream) : SIS3D_EUNSUPPORTED;
 }
 extern "C" int sis3d_conv3d_k3_tc_fused(const float *in, const float *w2_tc, const float *bias2, const float *w3_tc,
                                         const float *bias3, const float *residual, int res_ld, int res_coff, float *out,
                                         int out_ld, int out_coff, int X, int Y, int Z, int cin, int cmid, int cout, int act,
                                         void *stream) {
-    return conv3d_k3_tc_fused_impl(in, w2_tc, bias2, w3_tc, bias3, residual, res_ld, res_coff, out, out_ld, out_coff, X, Y, Z, cin,
-                                   cmid, cout, act, stream, 0);
+    return conv_tc_fused(TcFormat::TF32, in, w2_tc, bias2, w3_tc, bias3, residual, res_ld, res_coff, out, out_ld, out_coff, X, Y, Z,
+                         cin, cmid, cout, act, stream);
 }
 extern "C" int sis3d_conv3d_k3_tc_fused_x3(const float *in, const float *w2_x3, const float *bias2, const float *w3_x3,
                                            const float *bias3, const float *residual, int res_ld, int res_coff, float *out,
                                            int out_ld, int out_coff, int X, int Y, int Z, int cin, int cmid, int cout, int act,
                                            void *stream) {
-    return conv3d_k3_tc_fused_impl(in, w2_x3, bias2, w3_x3, bias3, residual, res_ld, res_coff, out, out_ld, out_coff, X, Y, Z, cin,
-                                   cmid, cout, act, stream, 1);
+    return conv_tc_fused(TcFormat::TF32X3, in, w2_x3, bias2, w3_x3, bias3, residual, res_ld, res_coff, out, out_ld, out_coff, X, Y,
+                         Z, cin, cmid, cout, act, stream);
 }
 extern "C" int sis3d_conv3d_k3_tc_fused_h3(const float *in, const uint16_t *w2_h3, const float *bias2, const uint16_t *w3_h3,
                                            const float *bias3, const float *residual, int res_ld, int res_coff, float *out,
                                            int out_ld, int out_coff, int X, int Y, int Z, int cin, int cmid, int cout, int act,
                                            void *stream) {
-    return conv3d_k3_tc_fused_impl(in, (const float *)w2_h3, bias2, (const float *)w3_h3, bias3, residual, res_ld, res_coff, out,
-                                   out_ld, out_coff, X, Y, Z, cin, cmid, cout, act, stream, 2);
+    return conv_tc_fused(TcFormat::F16X3, in, w2_h3, bias2, w3_h3, bias3, residual, res_ld, res_coff, out, out_ld, out_coff, X, Y,
+                         Z, cin, cmid, cout, act, stream);
 }
 
-// ---- y[M][N] = act(x[M][K] . w[N][K]^T + b): fully connected layer on the tensor cores (TF32), split-K ------------
+// ---- y[M][N] = act(x[M][K] . w[N][K]^T + b): fully connected layer on the tensor cores, split-K ------------------------------
 static int gemm_tc_splits(int M, int N, int K, int kc) {
     const int tiles = cdiv(M, TC_BM) * (N / (N >= 128 ? 128 : N));
     const int chunks = K / kc;
@@ -1055,154 +981,49 @@ extern "C" int sis3d_linear_tc_supported(int K, int N) { return (K % TC_KC == 0 
 extern "C" size_t sis3d_linear_tc_workspace_bytes(int M, int N, int K) {
     return sizeof(float) * (size_t)gemm_tc_splits(M, N, K, 16) * M * N + 16;  // the x3 variant splits K finer: covers both
 }
-static int linear_tc_impl(const float *x, const float *w_nk, const float *bias, float *y, int M, int K, int N, int act,
-                          void *workspace, size_t workspace_bytes, void *stream, int x3) {
+static int linear_tc(TcFormat fmt, const float *x, const void *w_nk, const float *bias, float *y, int M, int K, int N, int act,
+                     void *workspace, size_t workspace_bytes, void *stream) {
     if (!x || !w_nk || !y || !workspace || M <= 0) return SIS3D_EINVAL;
     if (!sis3d_linear_tc_supported(K, N)) return SIS3D_EUNSUPPORTED;
     if (((uintptr_t)x | (uintptr_t)w_nk | (uintptr_t)workspace) & 15) return SIS3D_EINVAL;
-    EncodeTiledFn enc = get_encode();
-    if (!enc) return SIS3D_EUNSUPPORTED;
-    const int BN = N >= 128 ? 128 : N;
-    const int kc = x3 == 1 ? 16 : TC_KC;
-    const CUtensorMapSwizzle sw = x3 == 1 ? CU_TENSOR_MAP_SWIZZLE_64B : CU_TENSOR_MAP_SWIZZLE_128B;
-    const CUtensorMapSwizzle swb = x3 == 1 ? CU_TENSOR_MAP_SWIZZLE_64B : CU_TENSOR_MAP_SWIZZLE_128B;
-    const CUtensorMapDataType dtb = x3 == 2 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT32;
-    int splits = gemm_tc_splits(M, N, K, kc);
-    const int chunks = K / kc;
+    if (!get_encode()) return SIS3D_EUNSUPPORTED;
+    const TcFormatInfo f = tc_format(fmt, K);
+    const int BN = min(N, f.bn_max);
+    int splits = gemm_tc_splits(M, N, K, f.kc);
+    const int chunks = K / f.kc;
     const int per = cdiv(chunks, splits);
     splits = cdiv(chunks, per);
     if (workspace_bytes < sizeof(float) * (size_t)splits * M * N) return SIS3D_EWORKSPACE;
     CUtensorMap tmA, tmB;
-    {
-        cuuint64_t dims[2] = {(cuuint64_t)K, (cuuint64_t)M};
-        cuuint64_t strides[1] = {(cuuint64_t)K * 4};
-        cuuint32_t box[2] = {(cuuint32_t)kc, TC_BM};
-        cuuint32_t estr[2] = {1, 1};
-        if (enc(&tmA, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, (void *)x, dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                sw, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) != CUDA_SUCCESS)
-            return SIS3D_EINVAL;
-        cuuint64_t dimsb[2] = {(cuuint64_t)K * (x3 == 2 ? 2 : 1), (cuuint64_t)N * (x3 == 1 ? 2 : 1)};
-        cuuint64_t stridesb[1] = {dimsb[0] * (x3 == 2 ? 2 : 4)};
-        cuuint32_t boxb[2] = {(cuuint32_t)(x3 == 2 ? 64 : kc), (cuuint32_t)BN};
-        if (enc(&tmB, dtb, 2, (void *)w_nk, dimsb, stridesb, boxb, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                swb, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) != CUDA_SUCCESS)
-            return SIS3D_EINVAL;
-    }
+    if (!encode_mat(&tmA, 4, x, K, M, f.kc, TC_BM, CU_TENSOR_MAP_L2_PROMOTION_L2_128B) ||
+        !encode_mat(&tmB, f.wb, w_nk, (int64_t)K * f.kmul, (int64_t)N * f.nmul, f.kc * f.kmul, BN, kWeightL2))
+        return SIS3D_EINVAL;
     TcArgs a = {};
     a.out = (float *)workspace; a.out_ld = N; a.cin = K; a.cout = N; a.gemm_m = M; a.gemm_chunks_per_split = per;
     cudaStream_t s = (cudaStream_t)stream;
-    const int mt = cdiv(M, TC_BM);
-    int rc;
-    if (x3 == 2) {
-        rc = BN == 32 ? launch_tc<32, 0, 4, 128, 2, 0, 2>(tmA, tmB, a, mt, s, nullptr, splits)
-           : BN == 64 ? launch_tc<64, 0, 4, 128, 2, 0, 2>(tmA, tmB, a, mt, s, nullptr, splits)
-                      : launch_tc<128, 0, 4, 128, 2, 0, 2>(tmA, tmB, a, mt, s, nullptr, splits);
-    } else if (x3) {
-        rc = BN == 32 ? launch_tc<32, 0, 4, 64, 2, 0, 1>(tmA, tmB, a, mt, s, nullptr, splits)
-           : BN == 64 ? launch_tc<64, 0, 4, 64, 2, 0, 1>(tmA, tmB, a, mt, s, nullptr, splits)
-                      : launch_tc<128, 0, 4, 64, 2, 0, 1>(tmA, tmB, a, mt, s, nullptr, splits);
-    } else {
-        rc = BN == 32 ? launch_tc<32, 0>(tmA, tmB, a, mt, s, nullptr, splits)
-           : BN == 64 ? launch_tc<64, 0>(tmA, tmB, a, mt, s, nullptr, splits)
-                      : launch_tc<128, 0>(tmA, tmB, a, mt, s, nullptr, splits);
-    }
+    const TcVariant *v = tc_variant(f, 0, BN, 2, 0);
+    const int rc = v ? v->launch(tmA, tmB, tmB, a, cdiv(M, TC_BM), splits, s) : SIS3D_EUNSUPPORTED;
     if (rc) return rc;
     gemm_splitk_reduce_kernel<<<cdiv(M * N, 256), 256, 0, s>>>((const float *)workspace, splits, (int64_t)M * N, bias, y, M, N, act);
     return finish_launch();
 }
 extern "C" int sis3d_linear_tc(const float *x, const float *w_nk, const float *bias, float *y, int M, int K, int N, int act,
                                void *workspace, size_t workspace_bytes, void *stream) {
-    return linear_tc_impl(x, w_nk, bias, y, M, K, N, act, workspace, workspace_bytes, stream, 0);
+    return linear_tc(TcFormat::TF32, x, w_nk, bias, y, M, K, N, act, workspace, workspace_bytes, stream);
 }
 // w_x3 = sis3d_pack_conv_weight_tc_x3(w[N][K] viewed as a 1x1 conv): [2][N][K]
 extern "C" int sis3d_linear_tc_x3(const float *x, const float *w_x3, const float *bias, float *y, int M, int K, int N, int act,
                                   void *workspace, size_t workspace_bytes, void *stream) {
-    return linear_tc_impl(x, w_x3, bias, y, M, K, N, act, workspace, workspace_bytes, stream, 1);
+    return linear_tc(TcFormat::TF32X3, x, w_x3, bias, y, M, K, N, act, workspace, workspace_bytes, stream);
 }
 extern "C" int sis3d_linear_tc_h3(const float *x, const uint16_t *w_h3, const float *bias, float *y, int M, int K, int N, int act,
                                   void *workspace, size_t workspace_bytes, void *stream) {
-    return linear_tc_impl(x, (const float *)w_h3, bias, y, M, K, N, act, workspace, workspace_bytes, stream, 2);
-}
-
-// ---- fp16-operand variant (kind::f16): activations and weights stored as fp16, fp32 accumulation in TMEM ----------
-extern "C" int sis3d_pack_conv_weight_tc_f16(const float *w, int cout, int cin, int ks, uint16_t *w16, void *stream) {
-    if (!w || !w16 || cout <= 0 || cin <= 0 || (ks != 1 && ks != 3)) return SIS3D_EINVAL;
-    const int taps = ks * ks * ks;
-    const int64_t total = (int64_t)cout * taps * cin;
-    pack_conv_weight_tc_f16_kernel<<<(int)imin64(cdiv64(total, 256), 148 * 8), 256, 0, (cudaStream_t)stream>>>(w, cout, cin, taps, (__half *)w16);
-    return finish_launch();
-}
-extern "C" int sis3d_cast_f16(const float *in, int in_ld, int in_coff, int64_t rows, int C, uint16_t *out, void *stream) {
-    if (!in || !out || rows <= 0 || C % 4 != 0 || (in_ld | in_coff) & 3) return SIS3D_EINVAL;
-    cast_f16_kernel<<<(int)imin64(cdiv64(rows * (C / 4), 256), 148 * 8), 256, 0, (cudaStream_t)stream>>>(in, in_ld, in_coff, rows, C / 4, (__half *)out);
-    return finish_launch();
-}
-extern "C" int sis3d_conv3d_tc_f16(const uint16_t *in16, const uint16_t *w16, const float *bias, const float *residual,
-                                   int res_ld, int res_coff, float *out32, uint16_t *out16, int out_ld, int out_coff, int X, int Y,
-                                   int Z, int cin, int cout, int ks, const int32_t *tiles, int n_tiles, int act, void *stream) {
-    if (!in16 || !w16 || (!out32 && !out16) || X <= 0 || Y <= 0 || Z <= 0 || (ks != 1 && ks != 3)) return SIS3D_EINVAL;
-    const int taps = ks * ks * ks;
-    if (!sis3d_conv3d_k3_tc_supported(cin, cout)) return SIS3D_EUNSUPPORTED;
-    if (((uintptr_t)in16 | (uintptr_t)w16 | (uintptr_t)out32 | (uintptr_t)out16) & 15) return SIS3D_EINVAL;
-    if ((out_ld | out_coff | res_ld | res_coff) & 3) return SIS3D_EINVAL;
-    EncodeTiledFn enc = get_encode();
-    if (!enc) return SIS3D_EUNSUPPORTED;
-    const bool wide = cin % 64 == 0;       // 64 channels = 128 B rows; C_in = 32 -> 64 B rows (SWIZZLE_64B)
-    const int BN = wide ? (cout >= 128 ? 128 : cout) : (cout >= 64 ? 64 : cout);  // 64-B rows: N tiles of at most 64
-    const int kc = wide ? 64 : 32;
-    if (!wide && cin != 32) return SIS3D_EUNSUPPORTED;
-    const int by = (tiles && ks == 3 && cout == 64 && wide) ? 4 : 2, bx = 16 / by;
-    const CUtensorMapSwizzle sw = wide ? CU_TENSOR_MAP_SWIZZLE_128B : CU_TENSOR_MAP_SWIZZLE_64B;
-    CUtensorMap tmA, tmB;
-    {
-        cuuint64_t dims[4] = {(cuuint64_t)cin, (cuuint64_t)Z, (cuuint64_t)Y, (cuuint64_t)X};
-        cuuint64_t strides[3] = {(cuuint64_t)cin * 2, (cuuint64_t)Z * cin * 2, (cuuint64_t)Y * Z * cin * 2};
-        cuuint32_t box[4] = {(cuuint32_t)kc, TC_BZ, (cuuint32_t)by, (cuuint32_t)(ks == 3 ? bx + 2 : bx)};
-        cuuint32_t estr[4] = {1, 1, 1, 1};
-        if (enc(&tmA, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 4, (void *)in16, dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, sw,
-                CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) != CUDA_SUCCESS)
-            return SIS3D_EINVAL;
-    }
-    {
-        cuuint64_t dims[2] = {(cuuint64_t)taps * cin, (cuuint64_t)cout};
-        cuuint64_t strides[1] = {(cuuint64_t)taps * cin * 2};
-        cuuint32_t box[2] = {(cuuint32_t)kc, (cuuint32_t)BN};
-        cuuint32_t estr[2] = {1, 1};
-        if (enc(&tmB, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 2, (void *)w16, dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, sw,
-                CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) != CUDA_SUCCESS)
-            return SIS3D_EINVAL;
-    }
-    TcArgs a = {};
-    a.bias = bias; a.res = residual; a.out = out32; a.out16 = (__half *)out16; a.tiles = tiles;
-    a.X = X; a.Y = Y; a.Z = Z; a.cin = cin; a.cout = cout; a.act = act;
-    a.out_ld = out_ld; a.out_coff = out_coff; a.res_ld = res_ld; a.res_coff = res_coff;
-    a.tiles_y = cdiv(Y, by); a.tiles_z = cdiv(Z, TC_BZ);
-    if (!tiles) n_tiles = cdiv(X, bx) * a.tiles_y * a.tiles_z;
-    if (n_tiles <= 0) return SIS3D_OK;
-    cudaStream_t s = (cudaStream_t)stream;
-    if (wide) {
-        if (ks == 3 && by == 4) return use_cluster() ? launch_tc<64, 3, 2, 128, 4, 0, 0, 2>(tmA, tmB, a, n_tiles, s)
-                                                     : launch_tc<64, 3, 2, 128, 4>(tmA, tmB, a, n_tiles, s);
-        if (ks == 3) {
-            switch (BN) {
-                case 32: return launch_tc<32, 3, 2, 128>(tmA, tmB, a, n_tiles, s);
-                case 64: return launch_tc<64, 3, 2, 128>(tmA, tmB, a, n_tiles, s);
-                default: return launch_tc<128, 3, 2, 128>(tmA, tmB, a, n_tiles, s);
-            }
-        }
-        switch (BN) {
-            case 32: return launch_tc<32, 1, 2, 128>(tmA, tmB, a, n_tiles, s);
-            case 64: return launch_tc<64, 1, 2, 128>(tmA, tmB, a, n_tiles, s);
-            default: return launch_tc<128, 1, 2, 128>(tmA, tmB, a, n_tiles, s);
-        }
-    }
-    if (ks == 3) return BN == 32 ? launch_tc<32, 3, 2, 64>(tmA, tmB, a, n_tiles, s) : launch_tc<64, 3, 2, 64>(tmA, tmB, a, n_tiles, s);
-    return BN == 32 ? launch_tc<32, 1, 2, 64>(tmA, tmB, a, n_tiles, s) : launch_tc<64, 1, 2, 64>(tmA, tmB, a, n_tiles, s);
+    return linear_tc(TcFormat::F16X3, x, w_h3, bias, y, M, K, N, act, workspace, workspace_bytes, stream);
 }
 
 // brick shape the tensor-core kernel uses for a layer (so callers can build matching tile lists)
 extern "C" void sis3d_conv3d_tc_brick(int with_tile_list, int ks, int cin, int cout, int32_t *bx, int32_t *by, int32_t *bz) {
-    const int y = (with_tile_list && ks == 3 && cout == 64 && cin % 64 == 0) ? 4 : 2;
+    const int y = tc_brick_y(with_tile_list != 0, ks, cin, cout);
     if (bx) *bx = 16 / y;
     if (by) *by = y;
     if (bz) *bz = TC_BZ;

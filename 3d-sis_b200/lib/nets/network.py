@@ -16,6 +16,7 @@ import gc
 import math
 import os
 import weakref
+from typing import NamedTuple, Optional
 
 import numpy as np
 import torch
@@ -97,6 +98,86 @@ class _MaskList:
         return list(self) == other if isinstance(other, list) else NotImplemented
 
 
+class Packed(NamedTuple):
+    """One layer's weights as the kernels take them."""
+    simt: torch.Tensor  # [k^3 C_in][ldw] for the CUDA-core kernels
+    bias: Optional[torch.Tensor]
+    cout: int
+    cin: int
+    ks: int
+    tc: dict  # tensor-core operand format ('tf32' | 'tf32x3' | 'f16x3' | 'fp16') -> packed weight
+
+
+# tensor-core operand format -> pack entry point, dtype, packed rows per output channel (tf32x3: hi rows, then lo rows;
+# f16x3: [32 hi | 32 lo] halves per 32-channel K slice, i.e. the same bytes as two fp16 rows)
+_TC_PACK = {"tf32": ("sis3d_pack_conv_weight_tc", torch.float32, 1),
+            "tf32x3": ("sis3d_pack_conv_weight_tc_x3", torch.float32, 2),
+            "f16x3": ("sis3d_pack_conv_weight_tc_h3", torch.float16, 2),
+            "fp16": ("sis3d_pack_conv_weight_tc_f16", torch.float16, 1)}
+# format -> entry point and timing label: convolutions (trailing arguments: the TF32 kernel also takes tile lists), fused
+# bottleneck tails, fully connected layers (+ workspace size query; None = the CUDA-core kernel)
+_CONV_TC = {"tf32": ("sis3d_conv3d_k3_tc", "conv_tc", (None, 0)),
+            "tf32x3": ("sis3d_conv3d_k3_tc_x3", "conv_tc_x3", ()),
+            "f16x3": ("sis3d_conv3d_k3_tc_h3", "conv_tc_h3", ())}
+_FUSED_TC = {"tf32": ("sis3d_conv3d_k3_tc_fused", "conv_tc_fused"),
+             "tf32x3": ("sis3d_conv3d_k3_tc_fused_x3", "conv_tc_fused_x3"),
+             "f16x3": ("sis3d_conv3d_k3_tc_fused_h3", "conv_tc_fused_h3")}
+_LINEAR = {None: ("sis3d_linear", "sis3d_linear_workspace_bytes", "linear"),
+           "tf32": ("sis3d_linear_tc", "sis3d_linear_tc_workspace_bytes", "linear_tc"),
+           "tf32x3": ("sis3d_linear_tc_x3", "sis3d_linear_tc_workspace_bytes", "linear_tc_x3"),
+           "f16x3": ("sis3d_linear_tc_h3", "sis3d_linear_tc_workspace_bytes", "linear_tc_h3")}
+
+
+# ---------------------------------------------------------------------------------------------------- conv routing
+def fp16_twins(math):
+    """Static stage: whether activations that feed tensor-core layers are kept as dense fp16 twins (and an fp32 copy only
+    where a consumer needs one), and the sparse back-projection writes one."""
+    return math == "fp16"
+
+
+def tc_format(math, formats, op="conv", tc_ok=True, out32=True, twin=False):
+    """Static stage: the tensor-core operand format a layer runs in, or None for the fp32 CUDA-core kernel.
+
+    math: the static-stage conv math; formats: the formats packed for the layer (for op 'fused', the bottleneck's conv2 +
+    conv3 in one kernel: those both convs have); tc_ok: geometry, input layout and activation fit the tensor-core kernel;
+    out32 / twin: the conv writes an fp32 output / an fp16 twin.  A conv in 'fp16' math without fp16 weights runs the TF32
+    kernel when it writes fp32 only; fully connected layers and fused tails have no fp16-operand kernel."""
+    if not tc_ok:
+        return None
+    if math in formats and (op == "conv" or math != "fp16"):
+        return math
+    if op == "conv" and math == "fp16" and "tf32" in formats and out32 and not twin:
+        return "tf32"
+    return None
+
+
+def mask_stage_code(mask_math, formats):
+    """The ragged mask stage's `math` (sis3d_mask_stage_launch): 2 = fp16-operand tensor cores on an fp16 canvas, 1 = TF32
+    tensor cores, 0 = CUDA-core; formats: those packed for mask_backbone.geometry.2."""
+    if mask_math == "fp16" and "tf32" in formats and "fp16" in formats:
+        return 2
+    return 1 if mask_math in ("tf32", "fp16") and "tf32" in formats else 0
+
+
+def _pack_tc(w, cout, cin, ks, formats):
+    """fp32 weight [cout][cin][ks][ks][ks] -> {format: packed tensor-core weight} for each of `formats`."""
+    out = {}
+    for f in formats:
+        sym, dtype, rows = _TC_PACK[f]
+        t = torch.empty(rows * cout, ks ** 3 * cin, dtype=dtype, device=w.device)
+        S.check(getattr(S.lib, sym)(S.ptr(w), cout, cin, ks, S.ptr(t), S.stream()), f"pack_{f}")
+        out[f] = t
+    return out
+
+
+def _conv_tc_formats(cin, cout, ks):
+    """Formats a 3-D convolution is packed in: fp16 storage needs 32 or a multiple of 64 input channels and has no 2x2x2
+    kernel."""
+    if ks not in (1, 2, 3) or not S.lib.sis3d_conv3d_k3_tc_supported(cin, cout):
+        return ()
+    return ("tf32", "tf32x3", "f16x3") + (("fp16",) if ks != 2 and (cin % 64 == 0 or cin == 32) else ())
+
+
 class Network(nn.Module):
     # layer programs of the concrete backbones are provided by subclasses (lib/nets/backbones.py)
     SPEC = None
@@ -105,15 +186,11 @@ class Network(nn.Module):
         super().__init__()
         self._predictions = {}
         self._feat_stride = [4, 4, 4]
-        self._packed = {}
+        self._packed = {}  # layer name -> Packed
         self._packed_version = None
         self._region_cache = {}
         self._const_cache = {}
         self._keep_debug = False
-        self._packed_tc = {}
-        self._packed_h = {}
-        self._packed_x3 = {}
-        self._packed_h3 = {}
         # conv math (see set_conv_math).  Default 'exact': error-compensated split products (fp32-class accuracy, tcgen05) in the
         # static stage -- everything that decides an integer output: proposal order, NMS keep list, class argmax, crop
         # bounds -- and fp16-stored operands in the ragged mask stage, whose outputs carry the 1e-3 tolerance.
@@ -292,7 +369,7 @@ class Network(nn.Module):
         self._pack_dirty = False
         if v == self._packed_version:
             return
-        self._packed, self._packed_tc, self._packed_h, self._packed_x3, self._packed_h3 = {}, {}, {}, {}, {}
+        self._packed = {}
         params = dict(self.named_parameters())
         self.__dict__["_enet"] = None
         if self.__dict__.get("_enet_names"):
@@ -311,29 +388,15 @@ class Network(nn.Module):
             ldw = (cout + 3) // 4 * 4
             packed = torch.empty(ks ** 3 * cin, ldw, dtype=torch.float32, device=w.device)
             S.check(S.lib.sis3d_pack_conv_weight(S.ptr(w), cout, cin, ks, S.ptr(packed), S.stream()), "pack")
+            if p.dim() == 5:
+                tc = _pack_tc(w, cout, cin, ks, _conv_tc_formats(cin, cout, ks))
+            elif cin >= 1024 and S.lib.sis3d_linear_tc_supported(cin, cout):
+                # nn.Linear [N][K] is already K-major for the TF32 GEMM; the split formats pack it as a 1x1 conv
+                tc = dict(tf32=p.detach(), **_pack_tc(w, cout, cin, 1, ("tf32x3", "f16x3")))
+            else:
+                tc = {}
             b = params.get(base + ".bias")
-            self._packed[base] = (packed, None if b is None else b.detach().float().contiguous(), cout, cin, ks)
-            if ks in (1, 2, 3) and p.dim() == 5 and S.lib.sis3d_conv3d_k3_tc_supported(cin, cout):
-                wtc = torch.empty(cout, ks ** 3 * cin, dtype=torch.float32, device=w.device)
-                S.check(S.lib.sis3d_pack_conv_weight_tc(S.ptr(w), cout, cin, ks, S.ptr(wtc), S.stream()), "pack_tc")
-                self._packed_tc[base] = wtc
-                wx3 = torch.empty(2 * cout, ks ** 3 * cin, dtype=torch.float32, device=w.device)
-                S.check(S.lib.sis3d_pack_conv_weight_tc_x3(S.ptr(w), cout, cin, ks, S.ptr(wx3), S.stream()), "pack_x3")
-                self._packed_x3[base] = wx3
-                wh3 = torch.empty(2 * cout, ks ** 3 * cin, dtype=torch.float16, device=w.device)
-                S.check(S.lib.sis3d_pack_conv_weight_tc_h3(S.ptr(w), cout, cin, ks, S.ptr(wh3), S.stream()), "pack_h3")
-                self._packed_h3[base] = wh3
-                if ks != 2 and (cin % 64 == 0 or cin == 32):
-                    w16 = torch.empty(cout, ks ** 3 * cin, dtype=torch.float16, device=w.device)
-                    S.check(S.lib.sis3d_pack_conv_weight_tc_f16(S.ptr(w), cout, cin, ks, S.ptr(w16), S.stream()), "pack_f16")
-                    self._packed_h[base] = w16
-            elif p.dim() == 2 and cin >= 1024 and S.lib.sis3d_linear_tc_supported(cin, cout):
-                wx3 = torch.empty(2 * cout, cin, dtype=torch.float32, device=w.device)  # nn.Linear [N][K] = a 1x1 conv
-                S.check(S.lib.sis3d_pack_conv_weight_tc_x3(S.ptr(w), cout, cin, 1, S.ptr(wx3), S.stream()), "pack_x3")
-                self._packed_x3[base] = wx3
-                wh3 = torch.empty(2 * cout, cin, dtype=torch.float16, device=w.device)
-                S.check(S.lib.sis3d_pack_conv_weight_tc_h3(S.ptr(w), cout, cin, 1, S.ptr(wh3), S.stream()), "pack_h3")
-                self._packed_h3[base] = wh3
+            self._packed[base] = Packed(packed, None if b is None else b.detach().float().contiguous(), cout, cin, ks, tc)
         for lvl in (1, 2, 3):  # both RPN heads of a level as ONE 1x1 conv: [2A | 6A] output channels, zero-padded to a
             # tensor-core friendly width (32/64/128k) so the merged head runs on the tcgen05 kernel as well
             c, b = f"rpn_cls_score_net_level{lvl}.0", f"rpn_bbox_pred_net_level{lvl}"
@@ -348,20 +411,8 @@ class Network(nn.Module):
                 bp[:cout] = bias
                 packed = torch.empty(cin, cpad, dtype=torch.float32, device=w.device)
                 S.check(S.lib.sis3d_pack_conv_weight(S.ptr(wp), cpad, cin, 1, S.ptr(packed), S.stream()), "pack")
-                self._packed[f"rpn_heads_level{lvl}"] = (packed, bp, cpad, cin, 1)
-                if S.lib.sis3d_conv3d_k3_tc_supported(cin, cpad):
-                    wtc = torch.empty(cpad, cin, dtype=torch.float32, device=w.device)
-                    S.check(S.lib.sis3d_pack_conv_weight_tc(S.ptr(wp), cpad, cin, 1, S.ptr(wtc), S.stream()), "pack_tc")
-                    self._packed_tc[f"rpn_heads_level{lvl}"] = wtc
-                    wx3 = torch.empty(2 * cpad, cin, dtype=torch.float32, device=w.device)
-                    S.check(S.lib.sis3d_pack_conv_weight_tc_x3(S.ptr(wp), cpad, cin, 1, S.ptr(wx3), S.stream()), "pack_x3")
-                    self._packed_x3[f"rpn_heads_level{lvl}"] = wx3
-                    wh3 = torch.empty(2 * cpad, cin, dtype=torch.float16, device=w.device)
-                    S.check(S.lib.sis3d_pack_conv_weight_tc_h3(S.ptr(wp), cpad, cin, 1, S.ptr(wh3), S.stream()), "pack_h3")
-                    self._packed_h3[f"rpn_heads_level{lvl}"] = wh3
-                    w16 = torch.empty(cpad, cin, dtype=torch.float16, device=w.device)
-                    S.check(S.lib.sis3d_pack_conv_weight_tc_f16(S.ptr(wp), cpad, cin, 1, S.ptr(w16), S.stream()), "pack_f16")
-                    self._packed_h[f"rpn_heads_level{lvl}"] = w16
+                self._packed[f"rpn_heads_level{lvl}"] = Packed(packed, bp, cpad, cin, 1,
+                                                               _pack_tc(wp, cpad, cin, 1, _conv_tc_formats(cin, cpad, 1)))
         torch.cuda.current_stream().synchronize()
         self._packed_version = v
         # captured graphs hold the addresses of the previous packed weights: drop them (re-captured on next use)
@@ -404,40 +455,39 @@ class Network(nn.Module):
             self._rec_end(tok)
         return x.h
 
-    def _conv(self, x: Act, name, stride=1, pad=None, act=0, residual: Act = None, out: Act = None,
-              regions=None, out_dims=None, want32=True, want16=False, out16=None):
-        """One convolution.  Dispatch: tcgen05 fp16-operand kernel ('fp16' math), tcgen05 TF32 kernel ('tf32'), else the
-        fp32 CUDA-core kernel.  want32/want16 choose which of the fp32 output / dense fp16 twin are produced (the twin
-        feeds the next tensor-core layer in 'fp16' math); out16 = caller-provided fp16 destination (ragged mask stage)."""
-        packed, bias, cout, cin, ks = self._packed[name]
+    def _conv(self, x: Act, name, stride=1, pad=None, act=0, residual: Act = None, out: Act = None, out_dims=None,
+              want32=True, want16=False):
+        """One convolution, on the kernel tc_format picks.  want32/want16 choose which of the fp32 output / dense fp16 twin
+        are produced where fp16_twins holds (the twin feeds the next tensor-core layer); elsewhere the output is fp32."""
+        r = self._packed[name]
+        cout, cin, ks = r.cout, r.cin, r.ks
         if cin != x.C:
             raise S.Sis3dError(f"{name}: expected {cin} input channels, got {x.C}")
         if pad is None:
             pad = 1 if ks == 3 else 0
         if out_dims is None:
             out_dims = tuple(d // 2 for d in x.dims) if stride == 2 else x.dims
-        regions_given = regions
         dev = (x.t if x.t is not None else x.h).device
-        f16 = self._math == "fp16"
         if ks == 2:  # the 2x2x2 / stride-2 downsampling convs run on the tensor cores too (element-strided TMA boxes)
             geom_ok = stride == 2 and pad == 0 and min(x.dims) >= 2 and self._tc_k2s2
         else:
             geom_ok = stride == 1 and pad == (1 if ks == 3 else 0)
-        tc_ok = (regions_given is None and geom_ok and x.layout == "vc" and x.ld == x.C and x.coff == 0 and act in (0, 1))
-        if not f16:
+        tc_ok = geom_ok and x.layout == "vc" and x.ld == x.C and x.coff == 0 and act in (0, 1)
+        if not fp16_twins(self._math):
             want32, want16 = True, False
         if out is None:
             t32 = torch.empty(*out_dims, cout, dtype=torch.float32, device=dev) if want32 else None
             out = Act(t32, out_dims, cout)
-        twin_ok = out.ld == cout and out.coff == 0  # the twin shares the geometry of the fp32 output
-        if want16 and twin_ok and out16 is None:
+        want16 = want16 and out.ld == cout and out.coff == 0  # the twin shares the geometry of the fp32 output
+        if want16:
             out.h = torch.empty(*out_dims, cout, dtype=torch.float16, device=dev)
-        h_ptr = S.ptr(out16) if out16 is not None else (S.ptr(out.h) if (want16 and twin_ok) else None)
+        h_ptr = S.ptr(out.h) if want16 else None
         res_args = (S.ptr(residual.t) if residual is not None else None, residual.ld if residual is not None else 0,
                     residual.coff if residual is not None else 0)
-        if f16 and tc_ok and name in self._packed_h:
+        fmt = tc_format(self._math, r.tc, "conv", tc_ok, out32=out.t is not None or not want16, twin=want16)
+        if fmt == "fp16":
             tok = self._rec(f"conv_tc16[{name}]")
-            S.check(S.lib.sis3d_conv3d_tc_f16(S.ptr(self._half(x)), S.ptr(self._packed_h[name]), S.ptr(bias), *res_args,
+            S.check(S.lib.sis3d_conv3d_tc_f16(S.ptr(self._half(x)), S.ptr(r.tc[fmt]), S.ptr(r.bias), *res_args,
                                               S.ptr(out.t) if out.t is not None else None, h_ptr, out.ld, out.coff, *x.dims,
                                               cin, cout, ks, None, 0, act, S.stream()), f"conv3d_tc_f16[{name}]")
             self._rec_end(tok)
@@ -446,30 +496,18 @@ class Network(nn.Module):
             raise S.Sis3dError(f"{name}: this layer needs the fp32 activation but only the fp16 twin was produced")
         if out.t is None and h_ptr is None:
             out.t = torch.empty(*out_dims, cout, dtype=torch.float32, device=dev)
-        if self._math in ("tf32x3", "f16x3") and tc_ok and name in self._packed_x3 and out.t is not None and h_ptr is None:
-            h3 = self._math == "f16x3"
-            tok = self._rec(f"conv_tc_{'h3' if h3 else 'x3'}[{name}]")
-            fn = S.lib.sis3d_conv3d_k3_tc_h3 if h3 else S.lib.sis3d_conv3d_k3_tc_x3
-            S.check(fn(S.ptr(x.t), S.ptr((self._packed_h3 if h3 else self._packed_x3)[name]), S.ptr(bias), *res_args,
-                       S.ptr(out.t), out.ld, out.coff, *x.dims, cin, cout, ks, act, S.stream()),
-                    f"conv3d_k3_tc_x3[{name}]")
+        if fmt is not None:
+            sym, label, tiles = _CONV_TC[fmt]
+            tok = self._rec(f"{label}[{name}]")
+            S.check(getattr(S.lib, sym)(S.ptr(x.t), S.ptr(r.tc[fmt]), S.ptr(r.bias), *res_args, S.ptr(out.t), out.ld, out.coff,
+                                        *x.dims, cin, cout, ks, *tiles, act, S.stream()), f"{sym}[{name}]")
             self._rec_end(tok)
             return out
-        if self._math in ("tf32", "fp16") and tc_ok and name in self._packed_tc and out.t is not None and h_ptr is None:
-            tok = self._rec(f"conv_tc[{name}]")
-            S.check(S.lib.sis3d_conv3d_k3_tc(S.ptr(x.t), S.ptr(self._packed_tc[name]), S.ptr(bias), *res_args,
-                                             S.ptr(out.t), out.ld, out.coff, *x.dims, cin, cout, ks, None, 0, act, S.stream()),
-                    f"conv3d_k3_tc[{name}]")
-            self._rec_end(tok)
-            return out
-        if regions is None:
-            regions, n_tiles = self._regions_single(x, out_dims, stride)
-        else:
-            regions, n_tiles = regions
+        regions, n_tiles = self._regions_single(x, out_dims, stride)
         in_sc = 1 if x.layout == "vc" else x.nvox
         xin = x.t if x.coff == 0 else x.t.reshape(-1)[x.coff:]
         tok = self._rec(f"conv[{name}]")
-        S.check(S.lib.sis3d_conv3d_ex(S.ptr(xin), C.c_int64(in_sc), S.ptr(packed), S.ptr(bias), *res_args,
+        S.check(S.lib.sis3d_conv3d_ex(S.ptr(xin), C.c_int64(in_sc), S.ptr(r.simt), S.ptr(r.bias), *res_args,
                                       S.ptr(out.t) if out.t is not None else None, h_ptr, out.ld, out.coff, S.ptr(regions),
                                       regions.numel() // S.REGION_BYTES, n_tiles, cin, cout, ks, stride, pad, act, S.stream()),
                 f"conv3d[{name}]")
@@ -477,34 +515,17 @@ class Network(nn.Module):
         return out
 
     def _linear(self, x, name, act):
-        """y = act(x W^T + b) through the split-K kernel (classifier MLP + heads)."""
-        packed, bias, cout, cin, _ = self._packed[name]
+        """y = act(x W^T + b) through a split-K kernel (classifier MLP + heads)."""
+        r = self._packed[name]
         M = x.shape[0]
-        y = torch.empty(M, cout, dtype=torch.float32, device=x.device)
-        if self._math in ("tf32x3", "f16x3") and name in self._packed_x3:
-            h3 = self._math == "f16x3"
-            nbytes = int(S.lib.sis3d_linear_tc_workspace_bytes(M, cout, cin))
-            ws = torch.empty(nbytes, dtype=torch.uint8, device=x.device)
-            tok = self._rec(f"linear_tc_{'h3' if h3 else 'x3'}[{name}]")
-            fn = S.lib.sis3d_linear_tc_h3 if h3 else S.lib.sis3d_linear_tc_x3
-            S.check(fn(S.ptr(x), S.ptr((self._packed_h3 if h3 else self._packed_x3)[name]), S.ptr(bias), S.ptr(y), M, cin, cout, act,
-                       S.ptr(ws), C.c_size_t(nbytes), S.stream()), f"linear_tc_x3[{name}]")
-            self._rec_end(tok)
-            return y
-        if self._math == "tf32" and cin >= 1024 and S.lib.sis3d_linear_tc_supported(cin, cout):
-            w_nk = dict(self.named_parameters())[name + ".weight"].detach()  # nn.Linear layout [N][K] is already K-major
-            nbytes = int(S.lib.sis3d_linear_tc_workspace_bytes(M, cout, cin))
-            ws = torch.empty(nbytes, dtype=torch.uint8, device=x.device)
-            tok = self._rec(f"linear_tc[{name}]")
-            S.check(S.lib.sis3d_linear_tc(S.ptr(x), S.ptr(w_nk), S.ptr(bias), S.ptr(y), M, cin, cout, act, S.ptr(ws),
-                                          C.c_size_t(nbytes), S.stream()), f"linear_tc[{name}]")
-            self._rec_end(tok)
-            return y
-        nbytes = int(S.lib.sis3d_linear_workspace_bytes(M, cout, cin))
+        y = torch.empty(M, r.cout, dtype=torch.float32, device=x.device)
+        fmt = tc_format(self._math, r.tc, "linear")
+        sym, ws_sym, label = _LINEAR[fmt]
+        nbytes = int(getattr(S.lib, ws_sym)(M, r.cout, r.cin))
         ws = torch.empty(nbytes, dtype=torch.uint8, device=x.device)
-        tok = self._rec(f"linear[{name}]")
-        S.check(S.lib.sis3d_linear(S.ptr(x), S.ptr(packed), S.ptr(bias), S.ptr(y), M, cin, cout, act, S.ptr(ws),
-                                   C.c_size_t(nbytes), S.stream()), f"linear[{name}]")
+        tok = self._rec(f"{label}[{name}]")
+        S.check(getattr(S.lib, sym)(S.ptr(x), S.ptr(r.tc[fmt] if fmt else r.simt), S.ptr(r.bias), S.ptr(y), M, r.cin, r.cout, act,
+                                    S.ptr(ws), C.c_size_t(nbytes), S.stream()), f"{label}[{name}]")
         self._rec_end(tok)
         return y
 
@@ -514,24 +535,21 @@ class Network(nn.Module):
         is a dense tensor, for the next block's first conv)."""
         y = self._conv(x, name + ".conv1", act=1, want32=False, want16=True)
         n2, n3 = name + ".conv2", name + ".conv3"
-        x3 = self._math in ("tf32x3", "f16x3")
-        h3 = self._math == "f16x3"
-        wt = self._packed_h3 if h3 else (self._packed_x3 if x3 else self._packed_tc)
-        if self._math in ("tf32", "tf32x3", "f16x3") and self._fuse_bneck and n2 in wt and n3 in wt and y.t is not None:
-            _, _, cmid, cin, _ = self._packed[n2]
-            cout = self._packed[n3][2]
-            if y.ld == y.C and y.coff == 0 and S.lib.sis3d_conv3d_k3_tc_fused_supported(cin, cmid, cout):
-                # conv2 + conv3 (+x, ReLU) in one tcgen05 kernel: the cmid-wide activation never leaves the SM
-                if out is None:
-                    out = Act(torch.empty(*y.dims, cout, dtype=torch.float32, device=y.t.device), y.dims, cout)
-                tok = self._rec(f"conv_tc_fused{'_h3' if h3 else '_x3' if x3 else ''}[{name}]")
-                fn = (S.lib.sis3d_conv3d_k3_tc_fused_h3 if h3 else S.lib.sis3d_conv3d_k3_tc_fused_x3 if x3
-                      else S.lib.sis3d_conv3d_k3_tc_fused)
-                S.check(fn(S.ptr(y.t), S.ptr(wt[n2]), S.ptr(self._packed[n2][1]),
-                           S.ptr(wt[n3]), S.ptr(self._packed[n3][1]), S.ptr(x.t), x.ld, x.coff, S.ptr(out.t), out.ld, out.coff, *y.dims, cin,
-                           cmid, cout, 1, S.stream()), f"conv3d_k3_tc_fused[{name}]")
-                self._rec_end(tok)
-                return out
+        r2, r3 = self._packed[n2], self._packed[n3]
+        fused_ok = (self._fuse_bneck and y.t is not None and y.ld == y.C and y.coff == 0
+                    and bool(S.lib.sis3d_conv3d_k3_tc_fused_supported(r2.cin, r2.cout, r3.cout)))
+        fmt = tc_format(self._math, r2.tc.keys() & r3.tc.keys(), "fused", fused_ok)
+        if fmt is not None:
+            # conv2 + conv3 (+x, ReLU) in one tcgen05 kernel: the cmid-wide activation never leaves the SM
+            if out is None:
+                out = Act(torch.empty(*y.dims, r3.cout, dtype=torch.float32, device=y.t.device), y.dims, r3.cout)
+            sym, label = _FUSED_TC[fmt]
+            tok = self._rec(f"{label}[{name}]")
+            S.check(getattr(S.lib, sym)(S.ptr(y.t), S.ptr(r2.tc[fmt]), S.ptr(r2.bias), S.ptr(r3.tc[fmt]), S.ptr(r3.bias),
+                                        S.ptr(x.t), x.ld, x.coff, S.ptr(out.t), out.ld, out.coff, *y.dims, r2.cin, r2.cout,
+                                        r3.cout, 1, S.stream()), f"{sym}[{name}]")
+            self._rec_end(tok)
+            return out
         y = self._conv(y, n2, act=1, want32=False, want16=True)
         return self._conv(y, n3, act=1, residual=x, out=out, want32=True, want16=True)
 
@@ -614,10 +632,11 @@ class Network(nn.Module):
         if (self._sparse_color and not self._keep_debug and first[0] == "k2s2" and feats.shape[1] % 16 == 0
                 and first[3] in (32, 64)):
             # fused + sparse: never materialise the back-projected volume (csrc/sparse.cu)
-            packed, _, cout, cin, _ = self._packed[f"color.{first[1]}"]
+            r = self._packed[f"color.{first[1]}"]
+            cout = r.cout
             od = tuple(d // 2 for d in dims)
             out = Act(torch.empty(*od, cout, dtype=torch.float32, device=dev), od, cout)
-            if self._math == "fp16":
+            if fp16_twins(self._math):
                 out.h = torch.empty(*od, cout, dtype=torch.float16, device=dev)
             feats = feats.contiguous()
             feats_t = torch.empty(feats.shape[0], w * h, feats.shape[1], dtype=torch.float32, device=dev)
@@ -625,7 +644,7 @@ class Network(nn.Module):
             ws = torch.empty(nbytes, dtype=torch.uint8, device=dev)
             tok = self._rec("backproject_conv_k2s2")
             S.check(S.lib.sis3d_backproject_conv_k2s2_ex(S.ptr(feats), S.ptr(feats_t), S.ptr(pix), S.ptr(pairs), S.ptr(n_pairs),
-                                                         feats.shape[0], feats.shape[1], w, h, *dims, S.ptr(packed), cout,
+                                                         feats.shape[0], feats.shape[1], w, h, *dims, S.ptr(r.simt), cout,
                                                          S.ptr(out.t), S.ptr(out.h), out.ld, 0, S.ptr(ws), C.c_size_t(nbytes),
                                                          S.stream()),
                     "backproject_conv_k2s2")
@@ -747,9 +766,9 @@ class Network(nn.Module):
         p2, p3 = self._packed["classifier.2"], self._packed["classifier.4"]
         pc, pb = self._packed["classifier_cls_score_net"], self._packed["classifier_bbox_pred_net"]
         tok = self._rec("mlp_tail")
-        S.check(S.lib.sis3d_mlp_tail(S.ptr(x1), R, p2[3], S.ptr(p2[0]), S.ptr(p2[1]), p2[2], S.ptr(p3[0]), S.ptr(p3[1]), p3[2],
-                                     S.ptr(pc[0]), S.ptr(pc[1]), pc[2], S.ptr(pb[0]), S.ptr(pb[1]), pb[2], S.ptr(cls_t),
-                                     S.ptr(box_t), S.stream()), "mlp_tail")
+        S.check(S.lib.sis3d_mlp_tail(S.ptr(x1), R, p2.cin, S.ptr(p2.simt), S.ptr(p2.bias), p2.cout, S.ptr(p3.simt), S.ptr(p3.bias),
+                                     p3.cout, S.ptr(pc.simt), S.ptr(pc.bias), pc.cout, S.ptr(pb.simt), S.ptr(pb.bias), pb.cout,
+                                     S.ptr(cls_t), S.ptr(box_t), S.stream()), "mlp_tail")
         self._rec_end(tok)
         cls_score, bbox_pred = Act(cls_t, (R, 1, 1), nc), Act(box_t, (R, 1, 1), nc * 6)
         if self._keep_debug:
@@ -765,14 +784,14 @@ class Network(nn.Module):
         and travel in ONE pinned H2D copy; all buffers come from a grow-only arena."""
         dev = scene_ncdhw.device
         X, Y, Z = (int(v) for v in scene_ncdhw.shape[2:])
-        ncls = self._packed["mask_backbone.geometry.10"][2]
-        use_tc = self._mask_math in ("tf32", "fp16") and "mask_backbone.geometry.2" in self._packed_tc
+        ncls = self._packed["mask_backbone.geometry.10"].cout
+        math = mask_stage_code(self._mask_math, self._packed["mask_backbone.geometry.2"].tc)
         det_host = np.ascontiguousarray(det_host[:n], dtype=np.float32)
         plan = S.MaskPlan()
         cap = self._arena["mask_tables_host"].numel() if "mask_tables_host" in self._arena else 1 << 18
         while True:
             stage = self._ws("mask_tables_host", cap, torch.uint8, dev, pinned=True)
-            rc = S.lib.sis3d_mask_plan_build(C.c_void_p(det_host.ctypes.data), n, X, Y, Z, ncls, 1 if use_tc else 0,
+            rc = S.lib.sis3d_mask_plan_build(C.c_void_p(det_host.ctypes.data), n, X, Y, Z, ncls, 1 if math else 0,
                                              C.c_void_p(stage.data_ptr()), C.c_size_t(stage.numel()), C.byref(plan))
             if rc == -3:  # SIS3D_EWORKSPACE: grow the pinned staging buffer and retry
                 cap = int(plan.bytes) * 2
@@ -786,16 +805,14 @@ class Network(nn.Module):
         host = stage.numpy()
         offs = host[plan.off_offs:plan.off_offs + 8 * (nk + 1)].view(np.int64).copy()
         sizes = host[plan.off_sizes:plan.off_sizes + 12 * nk].view(np.int32).reshape(nk, 3).copy()
-        math = 0 if not use_tc else (2 if (self._mask_math == "fp16" and "mask_backbone.geometry.2" in self._packed_h) else 1)
         cvox = int(plan.canvas[0]) * int(plan.canvas[1]) * int(plan.canvas[2])
         a = S.MaskStage()
         a.scene, a.X, a.Y, a.Z, a.ncls, a.math = scene_ncdhw.data_ptr(), X, Y, Z, ncls, math
-        a.w_first = self._packed["mask_backbone.geometry.0"][0].data_ptr()
-        a.w_last = self._packed["mask_backbone.geometry.10"][0].data_ptr()
-        table = (self._packed, self._packed_tc, self._packed_h)[math]
+        a.w_first = self._packed["mask_backbone.geometry.0"].simt.data_ptr()
+        a.w_last = self._packed["mask_backbone.geometry.10"].simt.data_ptr()
         for i, idx in enumerate((2, 4, 6, 8)):
-            w = table[f"mask_backbone.geometry.{idx}"]
-            a.w_mid[i] = (w[0] if math == 0 else w).data_ptr()
+            r = self._packed[f"mask_backbone.geometry.{idx}"]
+            a.w_mid[i] = (r.tc[("tf32", "fp16")[math - 1]] if math else r.simt).data_ptr()
         a.tables = self._ws("mask_tables", nbytes, torch.uint8, dev).data_ptr()
         a.canvas_bytes = 2 * 64 * (total * 4 if math == 0 else cvox * (2 if math == 2 else 4))
         a.canvas = self._ws("mask_canvas", a.canvas_bytes, torch.uint8, dev).data_ptr()
